@@ -12,6 +12,7 @@ timed on this box's host cores.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
                   [--blocks B]      # blocks per GPU (default 1048576 = BASELINE configs[1])
+                  [--dump-outputs DIR]   # the last timed step's outputs as .npy, to compare two builds
 
 Multi-GPU: one process per GPU (torchrun), contiguous block ranges per rank, no collective
 on the data path (SURVEY.md §8e); only the timing is all-reduced (max) over ranks.
@@ -688,6 +689,8 @@ def run_b200(args):
         r, o = chk.decompress_safe(c, BLOCK)
         if r != BLOCK or o != src[b * BLOCK:(b + 1) * BLOCK].cpu().numpy().tobytes():
             raise SystemExit("bench: CPU checker rejects a GPU-compressed block")
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, "" if world == 1 else f"_rank{rank}", nblk, bound, stride, clen, dres, comp, src)
 
     # ---- max over ranks (device time)
     tt = torch.tensor([t_step_ms, t_comp_ms, t_dec_ms], device=dev, dtype=torch.float64)
@@ -794,6 +797,23 @@ def run_b200(args):
         dist.barrier()
         dist.destroy_process_group()
     return 0
+
+
+def dump_outputs(out_dir, suffix, nblk, bound, stride, clen, dres, comp, dec):
+    """What the last timed step handed its caller, as float32 .npy files (every value is an integer below 2^24, so exact):
+    the compressed length of every block, the decompressor's return value (bytes read) for every block, and for a fixed
+    seeded sample of 64 blocks their compressed streams (zero past each stream's length, in slots of compressBound bytes)
+    and their decompressed bytes.  About 42 MB at the default 1 M blocks."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    pick = np.sort(np.random.default_rng(0).choice(nblk, size=min(64, nblk), replace=False))
+    lens = clen.cpu().numpy()
+    streams = comp.view(nblk, stride)[pick, :bound].cpu().numpy().astype(np.float32)
+    streams[np.arange(bound)[None, :] >= lens[pick][:, None]] = 0
+    arrays = {"compressed_lengths": lens, "decompress_results": dres.cpu().numpy(), "sample_block_index": pick,
+              "sample_compressed": streams, "sample_decompressed": dec.view(nblk, BLOCK)[pick].cpu().numpy()}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), a.astype(np.float32))
 
 
 def run_e2e(args, L, dev, host, rank, world):
@@ -927,7 +947,13 @@ def main():
     ap.add_argument("--frames", type=int, default=32, help="config 3: 64 MiB frames per GPU")
     ap.add_argument("--hc-blocks", type=int, default=1 << 18, help="config 4: 256 KiB blocks per GPU")
     ap.add_argument("--hc-seconds", type=int, default=60, help="config 4: time budget of the timed pass")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step computed to DIR/<name>.npy (float32; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     if args.impl == "reference":
         return run_reference(args)
     return run_b200(args)

@@ -47,15 +47,70 @@ def blocks(checker, big=True):
 
 
 def calgary_blocks(limit=4):
-    """64 KiB cuts of the Calgary files when the reference tree is present (dev container only)."""
-    base = "/root/reference/src/test-resources/calgary"
+    """64 KiB cuts of the Calgary files book1, geo and pic (the reference's src/test-resources/calgary, which LZ4Test.java
+    round-trips): the first `limit` (at most 4) of each file; geo is 102400 bytes long, so it has two.  Stored under
+    tests/golden: book1@0, geo@0, geo@65536 and pic@0 as the reference's own LZ4 streams in calgary_lz4.json (checked
+    against their recorded digests here), the next three cuts of book1 and of pic in calgary_cuts.xz."""
+    import base64
+    import hashlib
+    import json
+    import lzma
+    from oracle import oracle as O
+    assert limit <= 4
+    port = O.Port()
+    cuts = {}
+    for b in json.load(open(os.path.join(HERE, "golden", "calgary_lz4.json")))["blocks"]:
+        r, d = port.decompress_safe(base64.b64decode(b["fast_b64"]), b["len"])
+        assert r == b["len"] and hashlib.sha256(d).hexdigest() == b["sha256"], b["name"]
+        cuts[b["name"]] = d
+    extra = lzma.decompress(open(os.path.join(HERE, "golden", "calgary_cuts.xz"), "rb").read())
+    for k, name in enumerate(CALGARY_XZ_CUTS):
+        cuts[name] = extra[k * 65536:(k + 1) * 65536]
     out = []
-    if os.path.isdir(base):
-        for f in ("book1", "geo", "pic"):
-            data = open(os.path.join(base, f), "rb").read()
-            for i in range(0, min(len(data), limit * 65536), 65536):
-                out.append((f"{f}@{i}", data[i:i + 65536]))
+    for f, size in (("book1", 768771), ("geo", 102400), ("pic", 513216)):
+        for i in range(0, min(size, limit * 65536), 65536):
+            out.append((f"{f}@{i}", cuts[f"{f}@{i}"]))
     return out
+
+
+CALGARY_XZ_CUTS = [f"{f}@{k * 65536}" for f in ("book1", "pic") for k in (1, 2, 3)]     # tests/golden/calgary_cuts.xz, in order
+
+
+def codec_variants(c: bytes, n: int, rng: random.Random):
+    """(stream, capacity) pairs around a compressed block `c` of `n` bytes: capacities off by a little, a cut and an
+    extended stream, and 25 mutations (tests/test_oracle_pin.py's differential against the reference's decoders)"""
+    variants = [(c, n), (c, n - 1), (c, n + 1), (c, n + 64), (c, 0), (c[:-1], n), (c + b"\0", n)]
+    variants += [(m, rng.choice([n, n + 1, n + 70, max(0, n - 5)])) for m in mutate(c, rng, 25)]
+    return [(cc, cap) for cc, cap in variants if cc]
+
+
+def compress_caps(c: bytes):
+    """output capacities around the size of a compressed block `c`: the limitedOutput thresholds (lz4.c:1085-1088)"""
+    return (len(c) - 1, len(c), len(c) + 3, len(c) // 2)
+
+
+def frame_header_len(f: bytes) -> int:
+    """bytes of an LZ4 frame's header: magic, FLG, BD, the optional content size and dictionary ID, HC"""
+    return 7 + (8 if f[4] & 0x08 else 0) + (4 if f[4] & 0x01 else 0)
+
+
+class ReferenceFrames:
+    """LZ4F_compressFrame's frames (the reference's writer) for the inputs the tests use, rebuilt without the reference:
+    its frames differ from the restated writer's only in the header (it shrinks the block size ID to the input and
+    writes no content size of 0), so each is the reference's recorded header in front of the restated writer's blocks,
+    checked against the recorded digest of the reference's whole frame (tests/golden/ref_outputs.json)."""
+    kind = "reference"
+
+    def __init__(self, port, table):
+        self.port, self.table = port, table
+
+    def frame_compress(self, data, bs_code=7, flags=1) -> bytes:
+        import hashlib
+        e = self.table[f"{len(data)}/{bs_code}/{flags}"]
+        f = self.port.frame_compress(data, bs_code, flags)
+        g = bytes.fromhex(e["head"]) + f[frame_header_len(f):]
+        assert hashlib.sha256(g).hexdigest() == e["sha256"], (len(data), bs_code, flags)
+        return g
 
 
 def mutate(c: bytes, rng: random.Random, k: int):

@@ -1,6 +1,5 @@
 """Pins the CPU oracle (oracle/*.c restatements) to the reference: against the committed golden
-vectors produced by the reference's own C (tests/golden/kat.json, always), and against
-oracle/_ref directly when it is available.  CPU only."""
+vectors produced by the reference's own C (tests/golden/kat.json and ref_outputs.json).  CPU only."""
 import hashlib
 import json
 import os
@@ -75,44 +74,54 @@ def test_compress_bound(port):
     assert port.compress_bound(0x7E000001) == 0 and port.compress_bound(-1) == 0
 
 
-# ------------------------------------------------------------------ differential against oracle/_ref
-def test_ref_differential_codec(port, ref):
-    assert ref.version() == KAT["lz4_version"]
+# ------------------------------------------------------------------ differential against the reference's recorded outputs
+REF = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "ref_outputs.json")))
+
+
+def test_ref_differential_codec(port):
+    """the restated codec against what the reference's LZ4_compress_default / LZ4_decompress_safe / LZ4_decompress_fast
+    returned for the same blocks, capacities and corrupted streams (tests/golden/ref_outputs.json)"""
+    assert REF["lz4_version"] == KAT["lz4_version"]
     rng = random.Random(2)
+    items = corpus.blocks(port, big=False) + corpus.calgary_blocks(2)
+    assert [name for name, _ in items] == [e["name"] for e in REF["codec"]]
     bad = 0
-    for name, d in corpus.blocks(ref, big=False) + corpus.calgary_blocks(2):
-        c = ref.compress(d)
-        assert port.compress(d) == c, name
-        for cap in (len(c) - 1, len(c), len(c) + 3, len(c) // 2):
-            assert port.compress(d, cap) == ref.compress(d, cap), (name, cap)     # limitedOutput thresholds
-        n = len(d)
-        variants = [(c, n), (c, n - 1), (c, n + 1), (c, n + 64), (c, 0), (c[:-1], n), (c + b"\0", n)]
-        variants += [(m, rng.choice([n, n + 1, n + 70, max(0, n - 5)])) for m in corpus.mutate(c, rng, 25)]
-        for cc, cap in variants:
-            if not cc:
-                continue
-            a, b = port.decompress_safe(cc, cap), ref.decompress_safe(cc, cap)
-            bad += a != b
+    for (name, d), e in zip(items, REF["codec"]):
+        c = port.compress(d)
+        assert sha(c) == e["c_sha256"], name
+        for cap, want in zip(corpus.compress_caps(c), e["caps"]):
+            got = port.compress(d, cap)
+            assert (None if got is None else sha(got)) == want, (name, cap)     # limitedOutput thresholds
+        safe, fast, decoded = [], [], hashlib.sha256()
+        for cc, cap in corpus.codec_variants(c, len(d), rng):
+            r, out = port.decompress_safe(cc, cap)
+            safe.append(r); decoded.update(out)
             if cap >= 0:
-                a, b = port.decompress_fast(cc, cap), ref.decompress_fast(cc, cap)
-                bad += (a[0] != b[0]) or (b[0] >= 0 and a[1] != b[1])
+                r, out = port.decompress_fast(cc, cap)
+                fast.append(r)
+                if r >= 0:
+                    decoded.update(out)
+        bad += (safe != e["safe"]) + (fast != e["fast"]) + (decoded.hexdigest() != e["decoded_sha256"])
     assert bad == 0
 
 
-def test_ref_differential_frames(port, ref):
-    """frames written by the restatement decode with the reference's LZ4F_decompress and vice versa"""
+def test_ref_differential_frames(port):
+    """frames written by the restatement decode with the reference's LZ4F_decompress (its recorded verdict on these exact
+    bytes) and the reference's LZ4F_compressFrame frames (corpus.ReferenceFrames) decode with the restatement"""
+    frames = REF["frames"]
+    ref = corpus.ReferenceFrames(port, frames)
     for n in (0, 1, 100, 65536, 65537, 300000, 5 << 20):
-        data = ref.datagen(n, 0.5, 0.0, n & 0xFF).tobytes()
+        data = port.datagen(n, 0.5, 0.0, n & 0xFF).tobytes()
         for bs in (4, 7):
             for flags in (0, 1, 3, 5, 7):
+                e = frames[f"{n}/{bs}/{flags}"]
                 f = port.frame_compress(data, bs, flags)
-                r, out = ref.frame_decompress(f, n + 16)
-                assert r == n and out == data, (n, bs, flags)
+                assert sha(f) == e["port_sha256"] and e["ref_decodes"] == [n, sha(data)], (n, bs, flags)
                 g = ref.frame_compress(data, bs, flags)
                 r, out = port.frame_decompress(g, n + 16)
                 assert r == n and out == data, (n, bs, flags, r)
     # concatenated + skippable frames (LZ4FrameIOStreamTest.java:253-309, 378-426)
-    a, b = b"hello frame " * 1000, ref.datagen(70000, 0.5, 0.0, 1).tobytes()
+    a, b = b"hello frame " * 1000, port.datagen(70000, 0.5, 0.0, 1).tobytes()
     skip = bytes([0x50, 0x2A, 0x4D, 0x18, 4, 0, 0, 0, 1, 2, 3, 4])
     cat = port.frame_compress(a, 4, 1) + skip + ref.frame_compress(b, 5, 1)
     r, out = port.frame_decompress(cat, len(a) + len(b))
