@@ -5,6 +5,7 @@
 #include "../../include/b200lz4.h"
 #include "kernels.h"
 
+#include <algorithm>
 #include <atomic>
 #include <cstdio>
 #include <cstdlib>
@@ -56,33 +57,51 @@ static int ensure_device()
 }
 
 // ---------------------------------------------------------------------------------------------
+// A buffer that grows on demand, in device or in pinned host memory.  The old buffer is freed before the new one is
+// allocated.
+enum Mem { DEVICE, PINNED };
+struct Buf { uint8_t* p = nullptr; size_t cap = 0; };
+
+static int grow(Buf& b, Mem mem, size_t need, size_t grown)
+{
+    if (need <= b.cap) return 0;
+    if (b.p) CK(mem == PINNED ? cudaFreeHost(b.p) : cudaFree(b.p));
+    b.p = nullptr; b.cap = 0;
+    CK(mem == PINNED ? cudaHostAlloc(&b.p, grown, cudaHostAllocDefault) : cudaMalloc(&b.p, grown));
+    b.cap = grown;
+    return 0;
+}
+static size_t staging_size(size_t need) { return need + (need >> 2) + 4096; }
+
+// A slot's descriptor arrays, [total | soff | doff | xoff] u64 then [slen | dcap | res] i32, in either copy (pinned or device).
+struct Desc {
+    uint64_t *total, *soff, *doff, *xoff;
+    int32_t *slen, *dcap, *res;
+    void* hash;                                        // per-buffer digests of a hash batch
+};
+static Desc desc_view(uint8_t* base, size_t nb)
+{
+    uint64_t* const u = (uint64_t*)base + 2;          // total and its pad take 16 bytes
+    int32_t* const i = (int32_t*)(u + 3 * nb);
+    return Desc{ (uint64_t*)base, u, u + nb, u + 2 * nb,
+                 i, i + nb, i + 2 * nb,
+                 u + nb };                             // hash: a hash batch has no dst slots, its digests take doff's place
+}
+
 // A pipeline slot: one stream, device staging for a chunk of blocks and pinned descriptor arrays.
 struct Slot {
     cudaStream_t st = nullptr;
     cudaEvent_t done = nullptr;
-    uint8_t *d_src = nullptr, *d_dst = nullptr; size_t src_cap = 0, dst_cap = 0;
-    uint8_t* d_aux = nullptr; size_t aux_cap = 0;      // compacted output (compact_host only)
-    uint8_t* h_out = nullptr; size_t h_out_cap = 0;    // pinned bounce for scattered dst slots
-    bool scatter = false;                              // retire must copy h_out -> caller slots
+    Buf src, dst;                                      // device
+    Buf aux;                                           // device: compacted output (compact_host only)
+    Buf out;                                           // pinned bounce for scattered dst slots
+    bool scatter = false;                              // retire must copy out -> caller slots
     cudaEvent_t drained = nullptr; bool draining = false;
-    // descriptors: [total | soff | doff | xoff] u64, [slen | dcap | res] i32 — one pinned and one device copy
-    uint8_t *h_desc = nullptr, *d_desc = nullptr; size_t desc_blocks = 0;
+    Buf h_desc, d_desc; size_t desc_blocks = 0;        // descriptors: one pinned and one device copy
     size_t i0 = 0, i1 = 0;            // block range in flight
     bool busy = false;
-    uint64_t* h_total() const { return (uint64_t*)h_desc; }
-    uint64_t* h_soff() const { return (uint64_t*)h_desc + 2; }
-    uint64_t* h_doff() const { return h_soff() + desc_blocks; }
-    uint64_t* h_xoff() const { return h_soff() + 2 * desc_blocks; }
-    int32_t*  h_slen() const { return (int32_t*)(h_soff() + 3 * desc_blocks); }
-    int32_t*  h_dcap() const { return h_slen() + desc_blocks; }
-    int32_t*  h_res()  const { return h_slen() + 2 * desc_blocks; }
-    uint64_t* d_total() const { return (uint64_t*)d_desc; }
-    uint64_t* d_soff() const { return (uint64_t*)d_desc + 2; }
-    uint64_t* d_doff() const { return d_soff() + desc_blocks; }
-    uint64_t* d_xoff() const { return d_soff() + 2 * desc_blocks; }
-    int32_t*  d_slen() const { return (int32_t*)(d_soff() + 3 * desc_blocks); }
-    int32_t*  d_dcap() const { return d_slen() + desc_blocks; }
-    int32_t*  d_res()  const { return d_slen() + 2 * desc_blocks; }
+    Desc host() const { return desc_view(h_desc.p, desc_blocks); }
+    Desc dev() const { return desc_view(d_desc.p, desc_blocks); }
     static size_t desc_bytes(size_t nb) { return 16 + nb * (3 * 8 + 3 * 4); }
 };
 
@@ -95,8 +114,6 @@ static constexpr size_t CHUNK_BLOCKS = 1 << 16;
 struct Ctx {
     int device = -1;
     Slot slot[NSLOTS];
-    // one-block path
-    uint8_t* h_bounce = nullptr; size_t bounce_cap = 0;    // pinned: [src | dst]
     ~Ctx() { /* process teardown frees device memory; explicit frees would race CUDA shutdown */ }
 };
 
@@ -164,52 +181,32 @@ static int get_ctx(Ctx** out)
 // A pipeline call that fails half way (a CUDA error, or an argument error found at a later chunk) must not leave
 // chunks in flight: the next call on this thread would retire them into ITS result array with the old block indices.
 // The guard waits for whatever was queued and clears the slots' bookkeeping unless the call ran to completion.
-static void ctx_abandon(Ctx* c)
-{
-    for (int k = 0; k < NSLOTS; k++) {
-        Slot& s = c->slot[k];
-        if (s.busy || s.draining) cudaStreamSynchronize(s.st);       // result of the wait is irrelevant here
-        s.busy = false; s.draining = false; s.scatter = false;
-    }
-}
 struct PipelineGuard {
     Ctx* c; bool completed = false;
-    explicit PipelineGuard(Ctx* c_) : c(c_) {}
-    ~PipelineGuard() { if (!completed) ctx_abandon(c); }
+    ~PipelineGuard()
+    {
+        if (completed) return;
+        for (Slot& s : c->slot) {
+            if (s.busy || s.draining) cudaStreamSynchronize(s.st);       // result of the wait is irrelevant here
+            s.busy = false; s.draining = false; s.scatter = false;
+        }
+    }
 };
 
 static int slot_reserve(Slot& s, size_t src_bytes, size_t dst_bytes, size_t nblocks, size_t aux_bytes = 0)
 {
     if (s.draining) { CK(cudaEventSynchronize(s.drained)); s.draining = false; }
-    if (aux_bytes > s.aux_cap) {
-        if (s.d_aux) CK(cudaFree(s.d_aux));
-        s.aux_cap = 0; s.d_aux = nullptr;
-        size_t cap = aux_bytes + (aux_bytes >> 2) + 4096;
-        CK(cudaMalloc(&s.d_aux, cap)); s.aux_cap = cap;
+    int rc = grow(s.aux, DEVICE, aux_bytes, staging_size(aux_bytes));
+    if (!rc) rc = grow(s.src, DEVICE, src_bytes, staging_size(src_bytes));
+    if (!rc) rc = grow(s.dst, DEVICE, dst_bytes, staging_size(dst_bytes));
+    if (!rc && nblocks > s.desc_blocks) {
+        const size_t nb = (nblocks + (nblocks >> 1) + 64 + 1) & ~size_t(1);    // even: keeps the i32 arrays 8-byte aligned
+        s.desc_blocks = 0;
+        rc = grow(s.d_desc, DEVICE, Slot::desc_bytes(nb), Slot::desc_bytes(nb));
+        if (!rc) rc = grow(s.h_desc, PINNED, Slot::desc_bytes(nb), Slot::desc_bytes(nb));
+        if (!rc) s.desc_blocks = nb;
     }
-    if (src_bytes > s.src_cap) {
-        if (s.d_src) CK(cudaFree(s.d_src));
-        s.src_cap = 0; s.d_src = nullptr;
-        size_t cap = src_bytes + (src_bytes >> 2) + 4096;
-        CK(cudaMalloc(&s.d_src, cap)); s.src_cap = cap;
-    }
-    if (dst_bytes > s.dst_cap) {
-        if (s.d_dst) CK(cudaFree(s.d_dst));
-        s.dst_cap = 0; s.d_dst = nullptr;
-        size_t cap = dst_bytes + (dst_bytes >> 2) + 4096;
-        CK(cudaMalloc(&s.d_dst, cap)); s.dst_cap = cap;
-    }
-    if (nblocks > s.desc_blocks) {
-        if (s.d_desc) CK(cudaFree(s.d_desc));
-        if (s.h_desc) CK(cudaFreeHost(s.h_desc));
-        s.d_desc = nullptr; s.h_desc = nullptr; s.desc_blocks = 0;
-        size_t nb = nblocks + (nblocks >> 1) + 64;
-        nb = (nb + 1) & ~size_t(1);                    // keeps the i32 arrays 8-byte aligned
-        CK(cudaMalloc(&s.d_desc, Slot::desc_bytes(nb)));
-        CK(cudaHostAlloc(&s.h_desc, Slot::desc_bytes(nb), cudaHostAllocDefault));
-        s.desc_blocks = nb;
-    }
-    return 0;
+    return rc;
 }
 
 enum Op { OP_COMPRESS_FAST, OP_COMPRESS_HC, OP_DEC_SAFE, OP_DEC_FAST };
@@ -225,163 +222,165 @@ static cudaError_t launch_op(Op op, const BatchArgs& a, int param, cudaStream_t 
     }
 }
 
-// finish the slot's in-flight chunk: wait, hand the per-block results (and, for scattered dst
-// layouts, the bytes staged in the pinned bounce buffer) to the caller
-static int slot_retire(Slot& s, int32_t* result, uint8_t* dst_base = nullptr, const uint64_t* dst_off = nullptr,
-                       const int32_t* dst_cap = nullptr)
+static uint64_t nonneg(int32_t v) { return v > 0 ? (uint64_t)v : 0; }
+
+// A pipeline chunk: blocks [i0, i1), their source bytes [s_lo, s_hi) and destination slots [d_lo, d_hi).
+struct Chunk {
+    size_t i0, i1; uint64_t s_lo, s_hi, d_lo, d_hi;
+    size_t nb() const { return i1 - i0; }
+    size_t s_span() const { return (size_t)(s_hi - s_lo); }
+    size_t d_span() const { return (size_t)(d_hi - d_lo); }
+};
+
+// Cuts the chunk that starts at block i0: one block at least, otherwise at most CHUNK_BLOCKS blocks and CHUNK_SPAN bytes of
+// source and, when the blocks have destination slots (dst_off), of destination.  Blocks ascend in both, and destination
+// slots do not overlap.  A negative length or capacity spans no bytes; the kernel reports it as that block's error.
+static int cut_chunk(Chunk& ch, size_t i0, size_t n, const uint64_t* src_off, const int32_t* src_len,
+                     const uint64_t* dst_off, const int32_t* dst_cap, const char* order_error)
 {
-    if (!s.busy) return 0;
-    CK(cudaEventSynchronize(s.done));
-    memcpy(result + s.i0, s.h_res(), (s.i1 - s.i0) * sizeof(int32_t));
-    if (s.scatter && dst_base) {
-        const uint64_t d_lo = dst_off[s.i0];
-        for (size_t k = s.i0; k < s.i1; k++)
-            if (dst_cap[k] > 0) memcpy(dst_base + dst_off[k], s.h_out + (dst_off[k] - d_lo), (size_t)dst_cap[k]);
+    const uint64_t d0 = dst_off ? dst_off[i0] : 0;
+    ch = Chunk{ i0, i0, src_off[i0], src_off[i0], d0, d0 };
+    for (size_t i = i0; i < n && i - i0 < CHUNK_BLOCKS; i++) {
+        if (src_off[i] < ch.s_lo || (dst_off && dst_off[i] < ch.d_hi)) return fail_arg(order_error);
+        const uint64_t s_hi = std::max(ch.s_hi, src_off[i] + nonneg(src_len[i]));
+        const uint64_t d_hi = dst_off ? std::max(ch.d_hi, dst_off[i] + nonneg(dst_cap[i])) : 0;
+        if (i > i0 && (s_hi - ch.s_lo > CHUNK_SPAN || d_hi - ch.d_lo > CHUNK_SPAN)) break;
+        ch.s_hi = s_hi; ch.d_hi = d_hi; ch.i1 = i + 1;
     }
-    s.scatter = false;
-    s.busy = false;
     return 0;
 }
 
-// Host-buffer batch: chunk, stage, launch, copy back.  Blocks ascend in src and dst.
+// Writes the chunk's source descriptors and queues the descriptor and source copies; the caller has written its own
+// descriptors.  The source keeps its 16-byte phase on the device, so aligned inputs stay aligned.
+static int upload(Slot& s, const Chunk& ch, const uint8_t* src_base, const uint64_t* src_off, const int32_t* src_len)
+{
+    const size_t phase = (size_t)((uintptr_t)(src_base + ch.s_lo) & 15);
+    const Desc h = s.host();
+    for (size_t k = 0; k < ch.nb(); k++) {
+        h.soff[k] = src_off[ch.i0 + k] - ch.s_lo + phase;
+        h.slen[k] = src_len[ch.i0 + k];
+    }
+    CK(cudaMemcpyAsync(s.d_desc.p, s.h_desc.p, Slot::desc_bytes(s.desc_blocks), cudaMemcpyHostToDevice, s.st));
+    if (ch.s_span()) CK(cudaMemcpyAsync(s.src.p + phase, src_base + ch.s_lo, ch.s_span(), cudaMemcpyHostToDevice, s.st));
+    return 0;
+}
+
+// The 3-slot H2D / kernel / D2H pipeline under every host-buffer batch.  Chunks go round the slots.  Before a slot takes a
+// chunk, the one it holds is finished: wait for its `done`, then retire(s) hands its results to the caller.  stage(s, ch)
+// reserves staging and queues the chunk's copies and launches on s.st.  At the end every slot is finished and every
+// `drained` copy (started by a retire) awaited.  A call that fails half way drains what it queued (PipelineGuard).
+template <class Stage, class Retire>
+static int run_pipeline(size_t n, const uint64_t* src_off, const int32_t* src_len, const uint64_t* dst_off,
+                        const int32_t* dst_cap, const char* order_error, Stage stage, Retire retire)
+{
+    Ctx* c; int rc = get_ctx(&c); if (rc) return rc;
+    PipelineGuard guard{ c };
+    auto finish = [&](Slot& s) -> int {
+        if (!s.busy) return 0;
+        CK(cudaEventSynchronize(s.done));
+        const int r = retire(s); if (r) return r;
+        s.busy = false;
+        return 0;
+    };
+    int cur = 0;
+    for (size_t i0 = 0; i0 < n; cur = (cur + 1) % NSLOTS) {
+        Chunk ch;
+        rc = cut_chunk(ch, i0, n, src_off, src_len, dst_off, dst_cap, order_error); if (rc) return rc;
+        Slot& s = c->slot[cur];
+        rc = finish(s); if (rc) return rc;
+        rc = stage(s, ch); if (rc) return rc;
+        CK(cudaEventRecord(s.done, s.st));
+        s.busy = true; s.i0 = ch.i0; s.i1 = ch.i1;
+        i0 = ch.i1;
+    }
+    for (int k = 0; k < NSLOTS; k++) { rc = finish(c->slot[(cur + k) % NSLOTS]); if (rc) return rc; }
+    for (Slot& s : c->slot) if (s.draining) { CK(cudaEventSynchronize(s.drained)); s.draining = false; }
+    guard.completed = true;
+    return 0;
+}
+
+// Host-buffer batch of one codec op.  Blocks ascend in src and dst.
 static int host_batch(Op op, const uint8_t* src_base, const uint64_t* src_off, const int32_t* src_len,
                       uint8_t* dst_base, const uint64_t* dst_off, const int32_t* dst_cap,
                       int32_t* result, size_t n, int param)
 {
     if (n == 0) return 0;
     if (!src_base || !src_off || !src_len || !dst_base || !dst_off || !dst_cap || !result) return fail_arg("null pointer");
-    Ctx* c; int rc = get_ctx(&c); if (rc) return rc;
-    PipelineGuard guard(c);
-
-    size_t i0 = 0; int cur = 0;
-    while (i0 < n) {
-        // ---- pick the chunk [i0, i1): bounded block count and bounded src/dst spans
-        const uint64_t s_lo = src_off[i0], d_lo = dst_off[i0];
-        uint64_t s_hi = s_lo, d_hi = d_lo;
-        size_t i1 = i0;
-        while (i1 < n && i1 - i0 < CHUNK_BLOCKS) {
-            if (src_len[i1] < 0 || dst_cap[i1] < 0) {
-                // negative sizes are per-block errors in the reference (lz4.c:1324, 1953); let the kernel report them
-            }
-            const uint64_t se = src_off[i1] + (uint64_t)(src_len[i1] > 0 ? src_len[i1] : 0);
-            const uint64_t de = dst_off[i1] + (uint64_t)(dst_cap[i1] > 0 ? dst_cap[i1] : 0);
-            if (src_off[i1] < s_lo || dst_off[i1] < d_lo || (i1 > i0 && dst_off[i1] < d_hi))
-                return fail_arg("blocks must ascend and not overlap in dst");
-            const uint64_t ns = se > s_hi ? se : s_hi, nd = de > d_hi ? de : d_hi;
-            if (i1 > i0 && (ns - s_lo > CHUNK_SPAN || nd - d_lo > CHUNK_SPAN)) break;
-            s_hi = ns; d_hi = nd; i1++;
-        }
-        const size_t nb = i1 - i0, s_span = (size_t)(s_hi - s_lo), d_span = (size_t)(d_hi - d_lo);
-
-        Slot& s = c->slot[cur];
-        rc = slot_retire(s, result, dst_base, dst_off, dst_cap); if (rc) return rc;
-        rc = slot_reserve(s, s_span + 16, d_span + 16, nb); if (rc) return rc;
-
-        // keep the source's 16-byte phase so aligned inputs stay aligned on the device
-        const size_t s_phase = (size_t)((uintptr_t)(src_base + s_lo) & 15), d_phase = (size_t)((uintptr_t)(dst_base + d_lo) & 15);
+    auto stage = [&](Slot& s, const Chunk& ch) -> int {
+        const size_t nb = ch.nb(), d_span = ch.d_span();
+        int rc = slot_reserve(s, ch.s_span() + 16, d_span + 16, nb); if (rc) return rc;
+        const size_t d_phase = (size_t)((uintptr_t)(dst_base + ch.d_lo) & 15);
+        const Desc h = s.host(), d = s.dev();
         for (size_t k = 0; k < nb; k++) {
-            s.h_soff()[k] = src_off[i0 + k] - s_lo + s_phase;
-            s.h_doff()[k] = dst_off[i0 + k] - d_lo + d_phase;
-            s.h_slen()[k] = src_len[i0 + k];
-            s.h_dcap()[k] = dst_cap[i0 + k];
+            h.doff[k] = dst_off[ch.i0 + k] - ch.d_lo + d_phase;
+            h.dcap[k] = dst_cap[ch.i0 + k];
         }
-        CK(cudaMemcpyAsync(s.d_desc, s.h_desc, Slot::desc_bytes(s.desc_blocks), cudaMemcpyHostToDevice, s.st));
-        if (s_span) CK(cudaMemcpyAsync(s.d_src + s_phase, src_base + s_lo, s_span, cudaMemcpyHostToDevice, s.st));
-        BatchArgs a{ s.d_src, s.d_soff(), s.d_slen(), s.d_dst, s.d_doff(), s.d_dcap(), s.d_res(), nb };
+        rc = upload(s, ch, src_base, src_off, src_len); if (rc) return rc;
+        BatchArgs a{ s.src.p, d.soff, d.slen, s.dst.p, d.doff, d.dcap, d.res, nb };
         CK(launch_op(op, a, param, s.st));
-        CK(cudaMemcpyAsync(s.h_res(), s.d_res(), nb * sizeof(int32_t), cudaMemcpyDeviceToHost, s.st));
-        // copy back: when the dst slots are back to back (the normal layout) one DMA lands straight in
-        // the caller's memory; otherwise the span goes to a pinned bounce buffer and retire() scatters
-        // the slots, so caller bytes BETWEEN non-adjacent slots are never touched
-        bool contiguous = true;
-        {
-            uint64_t end = d_lo;
-            for (size_t k = 0; k < nb && contiguous; k++) {
-                if (dst_off[i0 + k] != end) contiguous = false;
-                end = dst_off[i0 + k] + (uint64_t)(dst_cap[i0 + k] > 0 ? dst_cap[i0 + k] : 0);
-            }
-        }
-        if (d_span && n == 1) {
+        CK(cudaMemcpyAsync(h.res, d.res, nb * sizeof(int32_t), cudaMemcpyDeviceToHost, s.st));
+        if (!d_span) return 0;
+        if (n == 1) {
             // one block per call (the JNI shim's shape): the caller's bytes behind the result stay untouched, like in the
             // reference (a decoder called with maxDestLen = "rest of my buffer" must not clobber what lies further along),
             // and no stale staging bytes of another call leave the device.  Costs one more round trip of a few bytes.
             CK(cudaStreamSynchronize(s.st));
-            const int32_t r = s.h_res()[0];
+            const int32_t r = h.res[0];
             const size_t produced = op == OP_DEC_FAST ? (r >= 0 ? d_span : 0) : (size_t)(r > 0 ? r : 0);
-            if (produced) CK(cudaMemcpyAsync(dst_base + d_lo, s.d_dst + d_phase, produced < d_span ? produced : d_span, cudaMemcpyDeviceToHost, s.st));
-        } else if (d_span) {
-            if (contiguous) {
-                CK(cudaMemcpyAsync(dst_base + d_lo, s.d_dst + d_phase, d_span, cudaMemcpyDeviceToHost, s.st));
-            } else {
-                if (d_span > s.h_out_cap) {
-                    if (s.h_out) CK(cudaFreeHost(s.h_out));
-                    s.h_out = nullptr; s.h_out_cap = 0;
-                    const size_t cap = d_span + (d_span >> 2) + 4096;
-                    CK(cudaHostAlloc(&s.h_out, cap, cudaHostAllocDefault)); s.h_out_cap = cap;
-                }
-                CK(cudaMemcpyAsync(s.h_out, s.d_dst + d_phase, d_span, cudaMemcpyDeviceToHost, s.st));
-                s.scatter = true;
-            }
+            if (produced) CK(cudaMemcpyAsync(dst_base + ch.d_lo, s.dst.p + d_phase, std::min(produced, d_span), cudaMemcpyDeviceToHost, s.st));
+            return 0;
         }
-        CK(cudaEventRecord(s.done, s.st));
-        s.busy = true; s.i0 = i0; s.i1 = i1;
-        i0 = i1; cur = (cur + 1) % NSLOTS;
-    }
-    for (int k = 0; k < NSLOTS; k++) { rc = slot_retire(c->slot[(cur + k) % NSLOTS], result, dst_base, dst_off, dst_cap); if (rc) return rc; }
-    guard.completed = true;
-    return 0;
+        // when the dst slots are back to back (the normal layout) one DMA lands straight in the caller's memory; otherwise
+        // the span goes to a pinned bounce buffer and retire scatters the slots, so caller bytes BETWEEN non-adjacent slots
+        // are never touched
+        bool contiguous = true;
+        uint64_t end = ch.d_lo;
+        for (size_t i = ch.i0; i < ch.i1 && contiguous; i++) {
+            contiguous = dst_off[i] == end;
+            end = dst_off[i] + nonneg(dst_cap[i]);
+        }
+        if (contiguous) {
+            CK(cudaMemcpyAsync(dst_base + ch.d_lo, s.dst.p + d_phase, d_span, cudaMemcpyDeviceToHost, s.st));
+        } else {
+            rc = grow(s.out, PINNED, d_span, staging_size(d_span)); if (rc) return rc;
+            CK(cudaMemcpyAsync(s.out.p, s.dst.p + d_phase, d_span, cudaMemcpyDeviceToHost, s.st));
+            s.scatter = true;
+        }
+        return 0;
+    };
+    auto retire = [&](Slot& s) -> int {
+        memcpy(result + s.i0, s.host().res, (s.i1 - s.i0) * sizeof(int32_t));
+        if (s.scatter) {
+            const uint64_t d_lo = dst_off[s.i0];
+            for (size_t k = s.i0; k < s.i1; k++)
+                if (dst_cap[k] > 0) memcpy(dst_base + dst_off[k], s.out.p + (dst_off[k] - d_lo), (size_t)dst_cap[k]);
+        }
+        s.scatter = false;
+        return 0;
+    };
+    return run_pipeline(n, src_off, src_len, dst_off, dst_cap, "blocks must ascend and not overlap in dst", stage, retire);
 }
 
 template <typename W>
-static int hash_host_batch(int bits, const uint8_t* base, const uint64_t* off, const int32_t* len, uint64_t seed,
+static int hash_host_batch(const uint8_t* base, const uint64_t* off, const int32_t* len, uint64_t seed,
                            W* out, size_t n)
 {
     if (n == 0) return 0;
     if (!base || !off || !len || !out) return fail_arg("null pointer");
-    Ctx* c; int rc = get_ctx(&c); if (rc) return rc;
-    PipelineGuard guard(c);
-    size_t i0 = 0; int cur = 0;
-    while (i0 < n) {
-        const uint64_t lo = off[i0]; uint64_t hi = lo; size_t i1 = i0;
-        while (i1 < n && i1 - i0 < CHUNK_BLOCKS) {
-            if (off[i1] < lo) return fail_arg("buffers must ascend");
-            const uint64_t e = off[i1] + (uint64_t)(len[i1] > 0 ? len[i1] : 0);
-            const uint64_t nh = e > hi ? e : hi;
-            if (i1 > i0 && nh - lo > CHUNK_SPAN) break;
-            hi = nh; i1++;
-        }
-        const size_t nb = i1 - i0, span = (size_t)(hi - lo);
-        Slot& s = c->slot[cur];
-        if (s.busy) {
-            CK(cudaEventSynchronize(s.done));
-            memcpy(out + s.i0, s.h_doff(), (s.i1 - s.i0) * sizeof(W));   // h_doff doubles as the pinned result area
-            s.busy = false;
-        }
-        rc = slot_reserve(s, span + 16, 16, nb); if (rc) return rc;
-        const size_t phase = (size_t)((uintptr_t)(base + lo) & 15);
-        for (size_t k = 0; k < nb; k++) { s.h_soff()[k] = off[i0 + k] - lo + phase; s.h_slen()[k] = len[i0 + k]; }
-        CK(cudaMemcpyAsync(s.d_desc, s.h_desc, Slot::desc_bytes(s.desc_blocks), cudaMemcpyHostToDevice, s.st));
-        if (span) CK(cudaMemcpyAsync(s.d_src + phase, base + lo, span, cudaMemcpyHostToDevice, s.st));
+    auto stage = [&](Slot& s, const Chunk& ch) -> int {
+        const size_t nb = ch.nb(), span = ch.s_span();
+        int rc = slot_reserve(s, span + 16, 16, nb); if (rc) return rc;
+        rc = upload(s, ch, base, off, len); if (rc) return rc;
+        const Desc d = s.dev();
+        const bool long_bufs = span / nb >= XXH_LONG_AVG;
         g_launches.fetch_add(1, std::memory_order_relaxed);
-        if (bits == 32) CK((span / nb >= 32768 ? launch_xxh32_long : launch_xxh32)(            // few long streams: one warp each
-                               s.d_src, s.d_soff(), s.d_slen(), (uint32_t)seed, (uint32_t*)s.d_doff(), nb, s.st));
-        else            CK((span / nb >= 32768 ? launch_xxh64_long : launch_xxh64)(
-                               s.d_src, s.d_soff(), s.d_slen(), seed, (uint64_t*)s.d_doff(), nb, s.st));
-        CK(cudaMemcpyAsync(s.h_doff(), s.d_doff(), nb * sizeof(W), cudaMemcpyDeviceToHost, s.st));
-        CK(cudaEventRecord(s.done, s.st));
-        s.busy = true; s.i0 = i0; s.i1 = i1;
-        i0 = i1; cur = (cur + 1) % NSLOTS;
-    }
-    for (int k = 0; k < NSLOTS; k++) {
-        Slot& s = c->slot[(cur + k) % NSLOTS];
-        if (s.busy) {
-            CK(cudaEventSynchronize(s.done));
-            memcpy(out + s.i0, s.h_doff(), (s.i1 - s.i0) * sizeof(W));
-            s.busy = false;
-        }
-    }
-    guard.completed = true;
-    return 0;
+        if (sizeof(W) == 4) CK((long_bufs ? launch_xxh32_long : launch_xxh32)(s.src.p, d.soff, d.slen, (uint32_t)seed, (uint32_t*)d.hash, nb, s.st));
+        else                CK((long_bufs ? launch_xxh64_long : launch_xxh64)(s.src.p, d.soff, d.slen, seed, (uint64_t*)d.hash, nb, s.st));
+        CK(cudaMemcpyAsync(s.host().hash, d.hash, nb * sizeof(W), cudaMemcpyDeviceToHost, s.st));
+        return 0;
+    };
+    auto retire = [&](Slot& s) -> int { memcpy(out + s.i0, s.host().hash, (s.i1 - s.i0) * sizeof(W)); return 0; };
+    return run_pipeline(n, off, len, nullptr, nullptr, "buffers must ascend", stage, retire);
 }
 
 // one block, host buffers: the n = 1 case of the host batch path
@@ -396,6 +395,17 @@ static int one_block(Op op, const char* src, int src_len, char* dst, int dst_cap
     int rc = host_batch(op, (const uint8_t*)src, &zero, &src_len, (uint8_t*)dst, &zero, &dst_cap, &res, 1, param);
     if (rc) return rc;
     return res;
+}
+
+// one buffer, host memory: the n = 1 case of the host hash batch
+template <typename W>
+static W one_hash(const void* input, size_t len, uint64_t seed)
+{
+    const uint64_t zero = 0; int32_t l = (int32_t)len; W out = 0; static const char dummy = 0;
+    tl_status = 0;
+    if (len > 0x7FFFFFFFu) { fail_arg("len > 2^31-1"); return 0; }
+    if (hash_host_batch<W>((const uint8_t*)(input ? input : &dummy), &zero, &l, seed, &out, 1)) return 0;
+    return out;
 }
 
 // Pin the calling WORKER thread to the CPUs of the NUMA node its GPU hangs off (sysfs: the PCI device's numa_node and the
@@ -558,33 +568,19 @@ int b200lz4_decompress_fast_bounded(const char* src, int srcAvail, char* dst, in
     return one_block(OP_DEC_FAST, src, srcAvail, dst, originalSize, 0);
 }
 
-uint32_t b200xxh32(const void* input, size_t len, uint32_t seed)
-{
-    const uint64_t zero = 0; int32_t l = (int32_t)len; uint32_t out = 0; static const char dummy = 0;
-    tl_status = 0;
-    if (len > 0x7FFFFFFFu) { fail_arg("len > 2^31-1"); return 0; }
-    if (hash_host_batch<uint32_t>(32, (const uint8_t*)(input ? input : &dummy), &zero, &l, seed, &out, 1)) return 0;
-    return out;
-}
-uint64_t b200xxh64(const void* input, size_t len, uint64_t seed)
-{
-    const uint64_t zero = 0; int32_t l = (int32_t)len; uint64_t out = 0; static const char dummy = 0;
-    tl_status = 0;
-    if (len > 0x7FFFFFFFu) { fail_arg("len > 2^31-1"); return 0; }
-    if (hash_host_batch<uint64_t>(64, (const uint8_t*)(input ? input : &dummy), &zero, &l, seed, &out, 1)) return 0;
-    return out;
-}
+uint32_t b200xxh32(const void* input, size_t len, uint32_t seed) { return one_hash<uint32_t>(input, len, seed); }
+uint64_t b200xxh64(const void* input, size_t len, uint64_t seed) { return one_hash<uint64_t>(input, len, seed); }
 
 // ---- streaming state: device-resident struct + a pinned staging area, one stream per handle
 struct StreamHandle {
-    int bits; int device; void* d_state; uint8_t* d_buf; size_t buf_cap; cudaStream_t st; void* h_out;
+    int bits; int device; void* d_state; Buf buf; cudaStream_t st; void* h_out;
 };
 static void* stream_create(int bits, uint64_t seed)
 {
     if (ensure_device()) return nullptr;
     StreamHandle* h = new (std::nothrow) StreamHandle();
     if (!h) return nullptr;
-    h->bits = bits; h->device = tl_device; h->d_buf = nullptr; h->buf_cap = 0;
+    h->bits = bits; h->device = tl_device;
     if (cudaStreamCreateWithFlags(&h->st, cudaStreamNonBlocking) != cudaSuccess ||
         cudaMalloc(&h->d_state, bits == 32 ? sizeof(Xxh32State) : sizeof(Xxh64State)) != cudaSuccess ||
         cudaHostAlloc(&h->h_out, 8, cudaHostAllocDefault) != cudaSuccess) { fail_cuda(cudaGetLastError(), "stream_create"); delete h; return nullptr; }
@@ -606,17 +602,14 @@ static int stream_update(void* hv, const void* input, size_t len)
     StreamHandle* h = (StreamHandle*)hv; if (!h) return fail_arg("null state");
     if (len == 0) return 0;
     CK(cudaSetDevice(h->device));
-    if (len > h->buf_cap) {
+    if (len > h->buf.cap) {
         CK(cudaStreamSynchronize(h->st));
-        if (h->d_buf) CK(cudaFree(h->d_buf));
-        h->d_buf = nullptr; h->buf_cap = 0;
-        size_t cap = len + (len >> 1) + 4096;
-        CK(cudaMalloc(&h->d_buf, cap)); h->buf_cap = cap;
+        const int rc = grow(h->buf, DEVICE, len, len + (len >> 1) + 4096); if (rc) return rc;
     }
-    CK(cudaMemcpyAsync(h->d_buf, input, len, cudaMemcpyHostToDevice, h->st));
+    CK(cudaMemcpyAsync(h->buf.p, input, len, cudaMemcpyHostToDevice, h->st));
     g_launches.fetch_add(1, std::memory_order_relaxed);
-    if (h->bits == 32) CK(launch_xxh32_stream((Xxh32State*)h->d_state, XXH_OP_UPDATE, 0, h->d_buf, len, h->st));
-    else               CK(launch_xxh64_stream((Xxh64State*)h->d_state, XXH_OP_UPDATE, 0, h->d_buf, len, h->st));
+    if (h->bits == 32) CK(launch_xxh32_stream((Xxh32State*)h->d_state, XXH_OP_UPDATE, 0, h->buf.p, len, h->st));
+    else               CK(launch_xxh64_stream((Xxh64State*)h->d_state, XXH_OP_UPDATE, 0, h->buf.p, len, h->st));
     CK(cudaStreamSynchronize(h->st));          // the caller may reuse `input` as soon as we return
     return 0;
 }
@@ -642,7 +635,7 @@ static void stream_free(void* hv)
     StreamHandle* h = (StreamHandle*)hv; if (!h) return;
     cudaSetDevice(h->device);
     cudaStreamSynchronize(h->st);
-    cudaFree(h->d_state); if (h->d_buf) cudaFree(h->d_buf); cudaFreeHost(h->h_out); cudaStreamDestroy(h->st);
+    cudaFree(h->d_state); if (h->buf.p) cudaFree(h->buf.p); cudaFreeHost(h->h_out); cudaStreamDestroy(h->st);
     delete h;
 }
 
@@ -778,9 +771,9 @@ int b200lz4_decompress_fast_batch_host(const uint8_t* src_base, const uint64_t* 
                                        int32_t* result, size_t n)
 { return host_batch(OP_DEC_FAST, src_base, src_off, src_avail, dst_base, dst_off, dst_len, result, n, 0); }
 int b200xxh32_batch_host(const uint8_t* base, const uint64_t* off, const int32_t* len, uint32_t seed, uint32_t* out, size_t n)
-{ return hash_host_batch<uint32_t>(32, base, off, len, seed, out, n); }
+{ return hash_host_batch<uint32_t>(base, off, len, seed, out, n); }
 int b200xxh64_batch_host(const uint8_t* base, const uint64_t* off, const int32_t* len, uint64_t seed, uint64_t* out, size_t n)
-{ return hash_host_batch<uint64_t>(64, base, off, len, seed, out, n); }
+{ return hash_host_batch<uint64_t>(base, off, len, seed, out, n); }
 
 int b200lz4_compress_fast_compact_host(const uint8_t* src_base, const uint64_t* src_off, const int32_t* src_len,
                                        uint8_t* dst_base, size_t dst_capacity, uint64_t* out_off,
@@ -789,63 +782,44 @@ int b200lz4_compress_fast_compact_host(const uint8_t* src_base, const uint64_t* 
     if (total) *total = 0;
     if (n == 0) return 0;
     if (!src_base || !src_off || !src_len || !dst_base || !out_off || !result) return fail_arg("null pointer");
-    Ctx* c; int rc = get_ctx(&c); if (rc) return rc;
-    PipelineGuard guard(c);
-    uint64_t running = 0;
-    // retire the slot's chunk: learn its packed size, start the payload copy at the running offset
-    auto retire = [&](Slot& s) -> int {
-        if (!s.busy) return 0;
-        CK(cudaEventSynchronize(s.done));
-        const uint64_t tot = *s.h_total();
-        if (running + tot > dst_capacity) return fail_arg("dst_capacity too small for the packed stream");
-        if (tot) CK(cudaMemcpyAsync(dst_base + running, s.d_aux, (size_t)tot, cudaMemcpyDeviceToHost, s.st));
-        CK(cudaEventRecord(s.drained, s.st)); s.draining = true;
-        const size_t nb = s.i1 - s.i0;
-        memcpy(result + s.i0, s.h_res(), nb * sizeof(int32_t));
-        for (size_t k = 0; k < nb; k++) out_off[s.i0 + k] = running + s.h_xoff()[k];
-        running += tot; s.busy = false;
-        return 0;
-    };
-    size_t i0 = 0; int cur = 0;
-    while (i0 < n) {
-        const uint64_t s_lo = src_off[i0]; uint64_t s_hi = s_lo, bound_sum = 0; size_t i1 = i0;
-        while (i1 < n && i1 - i0 < CHUNK_BLOCKS) {
-            if (src_off[i1] < s_lo) return fail_arg("blocks must ascend");
-            const uint64_t len = (uint64_t)(src_len[i1] > 0 ? src_len[i1] : 0);
-            const uint64_t se = src_off[i1] + len, ns = se > s_hi ? se : s_hi;
-            if (i1 > i0 && ns - s_lo > CHUNK_SPAN) break;
-            s_hi = ns; bound_sum += ((len + len / 255 + 16) + 15) & ~uint64_t(15); i1++;
-        }
-        const size_t nb = i1 - i0, s_span = (size_t)(s_hi - s_lo);
-        Slot& s = c->slot[cur];
-        rc = retire(s); if (rc) return rc;
-        rc = slot_reserve(s, s_span + 16, (size_t)bound_sum + 16, nb, (size_t)bound_sum + 16); if (rc) return rc;
-        const size_t s_phase = (size_t)((uintptr_t)(src_base + s_lo) & 15);
-        uint64_t slot_pos = 0;
+    // each block compresses into a slot of its aligned bound; the compaction kernel then packs the chunk's streams
+    auto stage = [&](Slot& s, const Chunk& ch) -> int {
+        const size_t nb = ch.nb();
+        uint64_t slots = 0;
+        for (size_t i = ch.i0; i < ch.i1; i++) slots += lz4_slot_bytes(src_len[i]);
+        int rc = slot_reserve(s, ch.s_span() + 16, (size_t)slots + 16, nb, (size_t)slots + 16); if (rc) return rc;
+        const Desc h = s.host(), d = s.dev();
+        uint64_t pos = 0;
         for (size_t k = 0; k < nb; k++) {
-            const uint64_t len = (uint64_t)(src_len[i0 + k] > 0 ? src_len[i0 + k] : 0);
-            const uint64_t bnd = len + len / 255 + 16;
-            s.h_soff()[k] = src_off[i0 + k] - s_lo + s_phase;
-            s.h_doff()[k] = slot_pos;
-            s.h_slen()[k] = src_len[i0 + k];
-            s.h_dcap()[k] = (int32_t)bnd;
-            slot_pos += (bnd + 15) & ~uint64_t(15);
+            h.doff[k] = pos;
+            h.dcap[k] = (int32_t)lz4_bound(src_len[ch.i0 + k]);
+            pos += lz4_slot_bytes(src_len[ch.i0 + k]);
         }
-        CK(cudaMemcpyAsync(s.d_desc, s.h_desc, Slot::desc_bytes(s.desc_blocks), cudaMemcpyHostToDevice, s.st));
-        if (s_span) CK(cudaMemcpyAsync(s.d_src + s_phase, src_base + s_lo, s_span, cudaMemcpyHostToDevice, s.st));
-        BatchArgs a{ s.d_src, s.d_soff(), s.d_slen(), s.d_dst, s.d_doff(), s.d_dcap(), s.d_res(), nb };
+        rc = upload(s, ch, src_base, src_off, src_len); if (rc) return rc;
+        BatchArgs a{ s.src.p, d.soff, d.slen, s.dst.p, d.doff, d.dcap, d.res, nb };
         CK(launch_op(OP_COMPRESS_FAST, a, max_src_len, s.st));
         g_launches.fetch_add(2, std::memory_order_relaxed);
-        CK(launch_compact(s.d_dst, s.d_doff(), s.d_res(), s.d_aux, s.d_xoff(), s.d_total(), nb, s.st));
-        CK(cudaMemcpyAsync(s.h_desc, s.d_desc, Slot::desc_bytes(s.desc_blocks), cudaMemcpyDeviceToHost, s.st));
-        CK(cudaEventRecord(s.done, s.st));
-        s.busy = true; s.i0 = i0; s.i1 = i1;
-        i0 = i1; cur = (cur + 1) % NSLOTS;
-    }
-    for (int k = 0; k < NSLOTS; k++) { rc = retire(c->slot[(cur + k) % NSLOTS]); if (rc) return rc; }
-    for (int k = 0; k < NSLOTS; k++) { Slot& s = c->slot[k]; if (s.draining) { CK(cudaEventSynchronize(s.drained)); s.draining = false; } }
+        CK(launch_compact(s.dst.p, d.doff, d.res, s.aux.p, d.xoff, d.total, nb, s.st));
+        CK(cudaMemcpyAsync(s.h_desc.p, s.d_desc.p, Slot::desc_bytes(s.desc_blocks), cudaMemcpyDeviceToHost, s.st));
+        return 0;
+    };
+    // the chunk's packed size is known: start the payload copy at the running offset
+    uint64_t running = 0;
+    auto retire = [&](Slot& s) -> int {
+        const Desc h = s.host();
+        const uint64_t tot = *h.total;
+        if (running + tot > dst_capacity) return fail_arg("dst_capacity too small for the packed stream");
+        if (tot) CK(cudaMemcpyAsync(dst_base + running, s.aux.p, (size_t)tot, cudaMemcpyDeviceToHost, s.st));
+        CK(cudaEventRecord(s.drained, s.st)); s.draining = true;
+        const size_t nb = s.i1 - s.i0;
+        memcpy(result + s.i0, h.res, nb * sizeof(int32_t));
+        for (size_t k = 0; k < nb; k++) out_off[s.i0 + k] = running + h.xoff[k];
+        running += tot;
+        return 0;
+    };
+    const int rc = run_pipeline(n, src_off, src_len, nullptr, nullptr, "blocks must ascend", stage, retire);
+    if (rc) return rc;
     if (total) *total = running;
-    guard.completed = true;
     return 0;
 }
 
@@ -880,7 +854,7 @@ int b200lz4_compress_fast_compact_host_multi(const uint8_t* src_base, const uint
         uint64_t acc = 0; int g = 0;
         for (size_t i = 0; i <= n; i++) {
             while (g <= ndev && i == n * (size_t)g / (size_t)ndev) base[(size_t)g++] = acc;
-            if (i < n) { const uint64_t len = (uint64_t)(src_len[i] > 0 ? src_len[i] : 0); acc += ((len + len / 255 + 16) + 15) & ~uint64_t(15); }
+            if (i < n) acc += lz4_slot_bytes(src_len[i]);
         }
         if (acc > dst_capacity) return fail_arg("dst_capacity must hold the aligned bounds of all blocks");
     }
@@ -903,14 +877,14 @@ int b200xxh32_batch_host_multi(const uint8_t* base, const uint64_t* off, const i
 {
     if (n == 0) return 0;
     if (!base || !off || !len || !out) return fail_arg("null pointer");
-    return run_sharded(n, devices, ndev, [&](size_t lo, size_t cnt) { return hash_host_batch<uint32_t>(32, base, off + lo, len + lo, seed, out + lo, cnt); });
+    return run_sharded(n, devices, ndev, [&](size_t lo, size_t cnt) { return hash_host_batch<uint32_t>(base, off + lo, len + lo, seed, out + lo, cnt); });
 }
 int b200xxh64_batch_host_multi(const uint8_t* base, const uint64_t* off, const int32_t* len, uint64_t seed,
                                uint64_t* out, size_t n, const int* devices, int ndev)
 {
     if (n == 0) return 0;
     if (!base || !off || !len || !out) return fail_arg("null pointer");
-    return run_sharded(n, devices, ndev, [&](size_t lo, size_t cnt) { return hash_host_batch<uint64_t>(64, base, off + lo, len + lo, seed, out + lo, cnt); });
+    return run_sharded(n, devices, ndev, [&](size_t lo, size_t cnt) { return hash_host_batch<uint64_t>(base, off + lo, len + lo, seed, out + lo, cnt); });
 }
 
 int b200lz4_context_count(void) { return g_contexts.load(std::memory_order_relaxed); }

@@ -8,6 +8,7 @@
 // payload work (block compression / decompression, every XXH32) goes through the batch entry points,
 // i.e. the CUDA kernels.  No hashing or codec arithmetic runs on the host.
 #include "../../include/b200lz4.h"
+#include "kernels.h"
 #include <cstdlib>
 #include <cstring>
 #include <vector>
@@ -26,7 +27,7 @@ static int compress_blocks(const uint8_t* src, const uint64_t* soff, const int32
     }
     std::vector<int32_t> ccap(nb);
     uint64_t acc = 0;
-    for (size_t i = 0; i < nb; i++) { coff[i] = acc; ccap[i] = slen[i] + slen[i] / 255 + 16; acc += ((uint64_t)ccap[i] + 15) & ~uint64_t(15); }
+    for (size_t i = 0; i < nb; i++) { coff[i] = acc; ccap[i] = (int32_t)b200::lz4_bound(slen[i]); acc += b200::lz4_slot_bytes(slen[i]); }
     if (acc > tmp_cap) return B200LZ4_E_ARG;
     return b200lz4_compress_hc_batch_host(src, soff, slen, tmp, coff, ccap.data(), clen, nb, hc_level);
 }

@@ -34,7 +34,6 @@ struct FrameRec {
     uint64_t out_off;                   // slot-layout start of this frame's content
     bool complete;                      // read up to its EndMark (and content checksum); false: the container breaks off inside it
 };
-static constexpr uint64_t XXH_LONG_AVG = 32768;     // average stream length from which a whole warp per stream wins
 
 struct BlockRec { uint64_t src_off; uint32_t size; bool raw; uint32_t checksum; bool has_checksum; size_t frame; uint64_t out_off; uint32_t cap; };
 

@@ -39,6 +39,8 @@ cudaError_t launch_xxh32_frames_chained(const uint8_t* slots, const uint64_t* bl
                                         uint32_t* out, size_t n, cudaStream_t st);
 cudaError_t launch_xxh64(const uint8_t* base, const uint64_t* off, const int32_t* len, uint64_t seed,
                          uint64_t* out, size_t n, cudaStream_t st);
+// average buffer length from which the one-warp-per-buffer kernels (launch_xxh*_long) win
+static constexpr uint64_t XXH_LONG_AVG = 32768;
 
 // streaming hash: one device-resident state per handle, updated by a single-warp kernel
 struct Xxh32State { uint64_t total; uint32_t v[4]; uint8_t mem[16]; uint32_t memsize; uint32_t seed; uint32_t digest; };
@@ -53,6 +55,11 @@ cudaError_t launch_xxh64_long(const uint8_t* base, const uint64_t* off, const in
 // prefix-sum compaction of variable-length outputs (compact_host path)
 cudaError_t launch_compact(const uint8_t* slots, const uint64_t* slot_off, const int32_t* lens,
                            uint8_t* out, uint64_t* out_off, uint64_t* total, size_t n, cudaStream_t st);
+
+// LZ4_compressBound (lz4.h:212) of one block, a negative length counting as 0, and the block's slot in the packed layouts
+// (compact_host staging, the HC container writers): the bound rounded up to 16 bytes.
+static inline uint64_t lz4_bound(int32_t len) { const uint64_t n = len > 0 ? (uint64_t)len : 0; return n + n / 255 + 16; }
+static inline uint64_t lz4_slot_bytes(int32_t len) { return (lz4_bound(len) + 15) & ~uint64_t(15); }
 
 extern std::atomic<unsigned long long> g_launch_count;      // launches made outside capi.cu (frame / container calls, any thread)
 

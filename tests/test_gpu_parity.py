@@ -351,6 +351,9 @@ def test_failed_pipeline_call_leaves_nothing_in_flight(b200):
     small = np.zeros(1000, dtype=np.uint8)
     with pytest.raises(b200.B200Error, match="dst_capacity"):
         b200.batch.compress_fast_compact_host(src, soff, slen, small, max_src_len=65536)
+    # found at the LAST chunk instead, while the payload copies of the earlier chunks are still draining
+    with pytest.raises(b200.B200Error, match="dst_capacity"):
+        b200.batch.compress_fast_compact_host(src, soff, slen, np.zeros(n * cl - 1, dtype=np.uint8), max_src_len=65536)
     # same thread, same streams: a short batch and then the full one must come back exact
     dst = np.zeros(n * cl + 64, dtype=np.uint8)
     ooff, olen, total = b200.batch.compress_fast_compact_host(src[:5 * bl], soff[:5], slen[:5], dst, max_src_len=65536)
