@@ -22,21 +22,19 @@
 
 namespace b200 {
 
-static std::atomic<unsigned long long> g_launches{0};
-std::atomic<unsigned long long> g_launch_count{0};      // launches made by frame.cu / containers.cu
+std::atomic<unsigned long long> g_launches{0};
 static thread_local char tl_err[256] = "";
 static thread_local int tl_status = 0;          // B200LZ4_E_* of the last value-returning call (hashes, digests) on this thread
 static thread_local int tl_device = -1;          // -1: not chosen yet (defaults to device 0)
 
-static int fail_cuda(cudaError_t e, const char* where)
+int fail_cuda(cudaError_t e, const char* where)
 {
     snprintf(tl_err, sizeof tl_err, "%s: %s", where, cudaGetErrorString(e));
     if (e == cudaErrorNoDevice || e == cudaErrorInsufficientDriver || e == cudaErrorInitializationError)
         return tl_status = B200LZ4_E_NODEVICE;
     return tl_status = B200LZ4_E_CUDA;
 }
-static int fail_arg(const char* what) { snprintf(tl_err, sizeof tl_err, "invalid argument: %s", what); return tl_status = B200LZ4_E_ARG; }
-#define CK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return fail_cuda(e_, #call); } while (0)
+int fail_arg(const char* what) { snprintf(tl_err, sizeof tl_err, "invalid argument: %s", what); return tl_status = B200LZ4_E_ARG; }
 
 static int ensure_device()
 {
@@ -888,7 +886,7 @@ int b200xxh64_batch_host_multi(const uint8_t* base, const uint64_t* off, const i
 }
 
 int b200lz4_context_count(void) { return g_contexts.load(std::memory_order_relaxed); }
-uint64_t b200lz4_launch_count(void) { return g_launches.load(std::memory_order_relaxed) + g_launch_count.load(std::memory_order_relaxed); }
-void     b200lz4_launch_count_reset(void) { g_launches.store(0, std::memory_order_relaxed); g_launch_count.store(0, std::memory_order_relaxed); }
+uint64_t b200lz4_launch_count(void) { return g_launches.load(std::memory_order_relaxed); }
+void     b200lz4_launch_count_reset(void) { g_launches.store(0, std::memory_order_relaxed); }
 
 } // extern "C"

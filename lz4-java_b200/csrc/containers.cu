@@ -9,27 +9,43 @@
 // i.e. the CUDA kernels.  No hashing or codec arithmetic runs on the host.
 #include "../../include/b200lz4.h"
 #include "kernels.h"
-#include <cstdlib>
 #include <cstring>
+#include <memory>
+#include <new>
 #include <vector>
 
 static inline void put32(uint8_t* p, uint32_t v) { p[0] = (uint8_t)v; p[1] = (uint8_t)(v >> 8); p[2] = (uint8_t)(v >> 16); p[3] = (uint8_t)(v >> 24); }
 static inline uint32_t get32(const uint8_t* p) { return p[0] | (p[1] << 8) | (p[2] << 16) | ((uint32_t)p[3] << 24); }
 
-// The writers' compressor argument (LZ4FrameOutputStream / LZ4BlockOutputStream take any LZ4Compressor): hc_level 0 = the fast
-// compressor, packed output; 1..17 = LZ4_compress_HC at that level into bound-sized slots.  coff/clen as *_compact_host.
-static int compress_blocks(const uint8_t* src, const uint64_t* soff, const int32_t* slen, uint8_t* tmp, size_t tmp_cap,
-                           uint64_t* coff, int32_t* clen, size_t nb, int max_src_len, int hc_level)
+// Both writers' blocks: [0, n) cut into bs-byte blocks and compressed with the writer's compressor argument (LZ4FrameOutputStream /
+// LZ4BlockOutputStream take any LZ4Compressor): hc_level 0 = the fast compressor, packed output; 1..17 = LZ4_compress_HC at that
+// level into bound-sized slots.  Then put(src_off, src_len, payload, size, raw) for each block in order; raw: stored as it is,
+// because compressing did not shrink it.
+template <class Put>
+static int write_blocks(const uint8_t* src, size_t n, size_t bs, int hc_level, Put put)
 {
-    if (hc_level <= 0) {
-        uint64_t total = 0;
-        return b200lz4_compress_fast_compact_host(src, soff, slen, tmp, tmp_cap, coff, clen, nb, max_src_len, &total);
+    const size_t nb = (n + bs - 1) / bs;
+    if (nb == 0) return 0;
+    std::vector<uint64_t> soff(nb), coff(nb);
+    std::vector<int32_t> slen(nb), ccap(nb), clen(nb);
+    size_t tmp_cap = 0;
+    for (size_t i = 0; i < nb; i++) {
+        soff[i] = i * bs; slen[i] = (int32_t)(n - i * bs < bs ? n - i * bs : bs);
+        coff[i] = tmp_cap; ccap[i] = (int32_t)b200::lz4_bound(slen[i]);         // HC: the block's slot (the fast compressor packs, setting coff)
+        tmp_cap += b200::lz4_slot_bytes(slen[i]);
     }
-    std::vector<int32_t> ccap(nb);
-    uint64_t acc = 0;
-    for (size_t i = 0; i < nb; i++) { coff[i] = acc; ccap[i] = (int32_t)b200::lz4_bound(slen[i]); acc += b200::lz4_slot_bytes(slen[i]); }
-    if (acc > tmp_cap) return B200LZ4_E_ARG;
-    return b200lz4_compress_hc_batch_host(src, soff, slen, tmp, coff, ccap.data(), clen, nb, hc_level);
+    std::unique_ptr<uint8_t[]> tmp(new (std::nothrow) uint8_t[tmp_cap]);
+    if (!tmp) return b200::fail_arg("out of host memory");
+    uint64_t total = 0;
+    const int rc = hc_level <= 0
+        ? b200lz4_compress_fast_compact_host(src, soff.data(), slen.data(), tmp.get(), tmp_cap, coff.data(), clen.data(), nb, bs <= 65536 ? 65536 : 0, &total)
+        : b200lz4_compress_hc_batch_host(src, soff.data(), slen.data(), tmp.get(), coff.data(), ccap.data(), clen.data(), nb, hc_level);
+    if (rc) return rc;
+    for (size_t i = 0; i < nb; i++) {
+        const bool raw = clen[i] <= 0 || clen[i] >= slen[i];
+        put(soff[i], slen[i], raw ? src + soff[i] : tmp.get() + coff[i], raw ? (uint32_t)slen[i] : (uint32_t)clen[i], raw);
+    }
+    return 0;
 }
 
 extern "C" {
@@ -44,9 +60,9 @@ size_t b200lz4f_compress_bound(size_t n, int bsCode)
 // flags: bit0 content checksum, bit1 block checksums, bit2 content size.  Returns bytes written or a negative code.
 int64_t b200lz4f_compress_host_hc(const uint8_t* src, size_t n, uint8_t* dst, size_t cap, int bsCode, int flags, int hc_level)
 {
-    if (bsCode < 4 || bsCode > 7) return B200LZ4_E_ARG;
+    if (bsCode < 4 || bsCode > 7) return b200::fail_arg("bsCode must be 4..7");
     if (cap < b200lz4f_compress_bound(n, bsCode)) return -9;
-    const size_t bs = (size_t)1 << (8 + 2 * bsCode), nb = (n + bs - 1) / bs;
+    const size_t bs = (size_t)1 << (8 + 2 * bsCode);
     size_t o = 0;
     put32(dst, 0x184D2204u); o = 4;
     const size_t hdr = o;
@@ -54,37 +70,30 @@ int64_t b200lz4f_compress_host_hc(const uint8_t* src, size_t n, uint8_t* dst, si
     dst[o++] = (uint8_t)(bsCode << 4);
     if (flags & 4) { put32(dst + o, (uint32_t)n); put32(dst + o + 4, (uint32_t)((uint64_t)n >> 32)); o += 8; }
     const uint32_t hh = b200xxh32(dst + hdr, o - hdr, 0);                        // descriptor checksum (:187)
-    if (hh == 0 && b200lz4_last_error()[0]) { /* a real zero hash is possible; device errors are caught below */ }
+    int st = b200lz4_last_status();
+    if (st) return st;
     dst[o++] = (uint8_t)((hh >> 8) & 0xFF);
-    if (nb) {
-        std::vector<uint64_t> soff(nb), coff(nb), poff(nb);
-        std::vector<int32_t> slen(nb), clen(nb), plen(nb);
-        for (size_t i = 0; i < nb; i++) { soff[i] = i * bs; slen[i] = (int32_t)((n - i * bs) < bs ? (n - i * bs) : bs); }
-        size_t tmp_cap = 0; for (size_t i = 0; i < nb; i++) tmp_cap += (size_t)slen[i] + slen[i] / 255 + 32;
-        uint8_t* tmp = (uint8_t*)malloc(tmp_cap ? tmp_cap : 1);
-        if (!tmp) return B200LZ4_E_ARG;
-        int rc = compress_blocks(src, soff.data(), slen.data(), tmp, tmp_cap, coff.data(), clen.data(), nb, bs <= 65536 ? 65536 : 0, hc_level);
-        if (rc) { free(tmp); return rc; }
-        for (size_t i = 0; i < nb; i++) {                                        // writeBlock (:199-235)
-            const bool raw = clen[i] <= 0 || clen[i] >= slen[i];                 // stored uncompressed when it does not shrink (:215-222)
-            const uint32_t sz = raw ? (uint32_t)slen[i] : (uint32_t)clen[i];
-            put32(dst + o, sz | (raw ? 0x80000000u : 0u)); o += 4;
-            memcpy(dst + o, raw ? src + soff[i] : tmp + coff[i], sz);
-            poff[i] = o; plen[i] = (int32_t)sz; o += sz;
-            if (flags & 2) o += 4;                                               // block checksum slot, filled below
-        }
-        free(tmp);
-        if (flags & 2) {
-            std::vector<uint32_t> sums(nb);
-            rc = b200xxh32_batch_host(dst, poff.data(), plen.data(), 0, sums.data(), nb);
-            if (rc) return rc;
-            for (size_t i = 0; i < nb; i++) put32(dst + poff[i] + plen[i], sums[i]);
-        }
+    std::vector<uint64_t> poff; std::vector<int32_t> plen;
+    int rc = write_blocks(src, n, bs, hc_level, [&](uint64_t, int32_t, const uint8_t* payload, uint32_t size, bool raw) {
+        put32(dst + o, size | (raw ? 0x80000000u : 0u)); o += 4;                 // writeBlock (:199-235), stored when it does not shrink (:215-222)
+        memcpy(dst + o, payload, size);
+        poff.push_back(o); plen.push_back((int32_t)size); o += size;
+        if (flags & 2) o += 4;                                                   // block checksum slot, filled below
+    });
+    if (rc) return rc;
+    if (flags & 2) {
+        std::vector<uint32_t> sums(poff.size());
+        rc = b200xxh32_batch_host(dst, poff.data(), plen.data(), 0, sums.data(), poff.size());
+        if (rc) return rc;
+        for (size_t i = 0; i < sums.size(); i++) put32(dst + poff[i] + plen[i], sums[i]);
     }
     put32(dst + o, 0); o += 4;                                                   // EndMark (:243-245)
     if (flags & 1) {
         if (n > 0x7FFFFFFFull) return -10;
-        put32(dst + o, b200xxh32(src, n, 0)); o += 4;                            // content checksum (:246-249)
+        const uint32_t h = b200xxh32(src, n, 0);                                 // content checksum (:246-249)
+        st = b200lz4_last_status();
+        if (st) return st;
+        put32(dst + o, h); o += 4;
     }
     return (int64_t)o;
 }
@@ -111,34 +120,24 @@ size_t b200lz4block_compress_bound(size_t n, int blockSize)
 
 int64_t b200lz4block_compress_host_hc(const uint8_t* src, size_t n, uint8_t* dst, size_t cap, int blockSize, int hc_level)
 {
-    if (blockSize < 64 || blockSize > (1 << 25)) return B200LZ4_E_ARG;
+    if (blockSize < 64 || blockSize > (1 << 25)) return b200::fail_arg("blockSize must be 64..2^25");
     if (cap < b200lz4block_compress_bound(n, blockSize)) return -9;
     const int level = lz4block_level(blockSize);
-    const size_t bs = (size_t)blockSize, nb = (n + bs - 1) / bs;
     size_t o = 0;
-    if (nb) {
-        std::vector<uint64_t> soff(nb), coff(nb);
-        std::vector<int32_t> slen(nb), clen(nb);
-        std::vector<uint32_t> sums(nb);
-        for (size_t i = 0; i < nb; i++) { soff[i] = i * bs; slen[i] = (int32_t)((n - i * bs) < bs ? (n - i * bs) : bs); }
-        size_t tmp_cap = 0; for (size_t i = 0; i < nb; i++) tmp_cap += (size_t)slen[i] + slen[i] / 255 + 32;
-        uint8_t* tmp = (uint8_t*)malloc(tmp_cap ? tmp_cap : 1);
-        if (!tmp) return B200LZ4_E_ARG;
-        int rc = compress_blocks(src, soff.data(), slen.data(), tmp, tmp_cap, coff.data(), clen.data(), nb, bs <= 65536 ? 65536 : 0, hc_level);
-        if (!rc) rc = b200xxh32_batch_host(src, soff.data(), slen.data(), LZ4BLOCK_SEED, sums.data(), nb);   // checksum of the ORIGINAL bytes
-        if (rc) { free(tmp); return rc; }
-        for (size_t i = 0; i < nb; i++) {                                        // flushBufferedData (:203-227)
-            const bool raw = clen[i] <= 0 || clen[i] >= slen[i];
-            const uint32_t sz = raw ? (uint32_t)slen[i] : (uint32_t)clen[i];
-            memcpy(dst + o, LZ4BLOCK_MAGIC, 8);
-            dst[o + 8] = (uint8_t)((raw ? METHOD_RAW : METHOD_LZ4) | level);
-            put32(dst + o + 9, sz); put32(dst + o + 13, (uint32_t)slen[i]);
-            put32(dst + o + 17, sums[i] & 0x0FFFFFFFu);                          // Checksum view keeps 28 bits (StreamingXXHash32.java:106)
-            memcpy(dst + o + LZ4BLOCK_HEADER, raw ? src + soff[i] : tmp + coff[i], sz);
-            o += LZ4BLOCK_HEADER + sz;
-        }
-        free(tmp);
-    }
+    std::vector<uint64_t> soff, sum_at; std::vector<int32_t> slen;
+    int rc = write_blocks(src, n, (size_t)blockSize, hc_level, [&](uint64_t src_off, int32_t src_len, const uint8_t* payload, uint32_t size, bool raw) {
+        memcpy(dst + o, LZ4BLOCK_MAGIC, 8);                                      // flushBufferedData (:203-227)
+        dst[o + 8] = (uint8_t)((raw ? METHOD_RAW : METHOD_LZ4) | level);
+        put32(dst + o + 9, size); put32(dst + o + 13, (uint32_t)src_len);
+        memcpy(dst + o + LZ4BLOCK_HEADER, payload, size);
+        soff.push_back(src_off); slen.push_back(src_len); sum_at.push_back(o + 17);   // checksum slot, filled below
+        o += LZ4BLOCK_HEADER + size;
+    });
+    if (rc) return rc;
+    std::vector<uint32_t> sums(soff.size());
+    rc = b200xxh32_batch_host(src, soff.data(), slen.data(), LZ4BLOCK_SEED, sums.data(), soff.size());   // checksum of the ORIGINAL bytes
+    if (rc) return rc;
+    for (size_t i = 0; i < sums.size(); i++) put32(dst + sum_at[i], sums[i] & 0x0FFFFFFFu);   // Checksum view keeps 28 bits (StreamingXXHash32.java:106)
     memcpy(dst + o, LZ4BLOCK_MAGIC, 8);                                          // finish(): empty block (:255-266)
     dst[o + 8] = (uint8_t)(METHOD_RAW | level);
     put32(dst + o + 9, 0); put32(dst + o + 13, 0); put32(dst + o + 17, 0);

@@ -17,6 +17,7 @@
 #include "kernels.h"
 #include <cstring>
 #include <new>
+#include <type_traits>
 #include <vector>
 
 namespace b200 {
@@ -42,21 +43,43 @@ struct FrameIndex {
     std::vector<BlockRec> blocks;
     uint64_t slot_bytes = 0;            // device bytes needed for the slot layout (upper bound of the decoded size)
     int tail_err = 0;                   // the container's own error, behind everything indexed (reported after what precedes it)
-    // device-side descriptor arrays, built once
+    std::vector<size_t> comp_ix, raw_ix, bsum_ix, fsum_ix;      // compressed / stored blocks, blocks and frames with a checksum
+    std::vector<uint8_t> h_blob;        // the descriptor arrays (FrameDesc), built once
+    // device state, all of it on `device` or none of it (create_device_state / release_device_state)
     int device = -1;
-    uint8_t* d_blob = nullptr; size_t blob_bytes = 0;
-    std::vector<uint8_t> h_blob;
-    // offsets inside the blob
-    size_t o_c_soff, o_c_doff, o_c_slen, o_c_dcap, o_c_res;          // compressed blocks
-    size_t o_r_soff, o_r_doff, o_r_len;                              // raw blocks
-    size_t o_h_off, o_h_len, o_h_out;                                // header descriptors
-    size_t o_b_off, o_b_len, o_b_out;                                // block checksums
-    size_t o_f_first, o_f_nblk, o_f_out;                                        // content checksums (chained to the decoder: xxhash.cu)
-    size_t o_k_comp, o_k_rawlen, o_k_off;                            // per block: index among the compressed blocks (-1: stored), stored size, slot
+    uint8_t* d_blob = nullptr;          // the device copy of h_blob
     cudaStream_t st2 = nullptr; cudaEvent_t e1 = nullptr, e2 = nullptr;   // the checksum warps run beside the decoder
-    size_t n_comp = 0, n_raw = 0, n_bsum = 0, n_fsum = 0;
-    std::vector<size_t> comp_ix, raw_ix, bsum_ix, fsum_ix;
 };
+
+// The descriptor arrays of an index, in its host blob or in the device copy: every array starts on 16 bytes.
+struct FrameDesc {
+    uint64_t *c_soff, *c_doff; int32_t *c_slen, *c_dcap, *c_res;        // compressed blocks
+    uint64_t *r_soff, *r_doff; int32_t *r_len;                          // stored blocks
+    uint64_t *h_off; int32_t *h_len; uint32_t *h_out;                   // frame descriptors (header checksums)
+    uint64_t *b_off; int32_t *b_len; uint32_t *b_out;                   // block checksums
+    uint32_t *f_first, *f_nblk, *f_out;                                 // content checksums (chained to the decoder: xxhash.cu)
+    int32_t *k_comp, *k_rawlen; uint64_t *k_off;                        // per block: index among the compressed blocks (-1: stored), stored size, slot
+};
+// base == nullptr only measures the layout: *bytes receives the blob's size.
+static FrameDesc desc_view(uint8_t* base, const FrameIndex& ix, size_t* bytes = nullptr)
+{
+    const size_t nc = ix.comp_ix.size(), nr = ix.raw_ix.size(), nbs = ix.bsum_ix.size(), nfs = ix.fsum_ix.size();
+    const size_t nf = ix.frames.size(), nb = ix.blocks.size();
+    size_t o = 0;
+    auto take = [&](auto*& p, size_t count) {
+        p = base ? reinterpret_cast<std::remove_reference_t<decltype(p)>>(base + o) : nullptr;
+        o = (o + count * sizeof *p + 15) & ~size_t(15);
+    };
+    FrameDesc d;
+    take(d.c_soff, nc); take(d.c_doff, nc); take(d.c_slen, nc); take(d.c_dcap, nc); take(d.c_res, nc);
+    take(d.r_soff, nr); take(d.r_doff, nr); take(d.r_len, nr);
+    take(d.h_off, nf); take(d.h_len, nf); take(d.h_out, nf);
+    take(d.b_off, nbs); take(d.b_len, nbs); take(d.b_out, nbs);
+    take(d.f_first, nfs); take(d.f_nblk, nfs); take(d.f_out, nfs);
+    take(d.k_comp, nb); take(d.k_rawlen, nb); take(d.k_off, nb);
+    if (bytes) *bytes = o;
+    return d;
+}
 
 // LZ4FrameInputStream.nextFrameInfo / readHeader / readBlock as a pure index pass.  The reader is a stream: it hands out the
 // bytes of every frame before a malformed spot and fails THERE, after any checksum or decode error that lies earlier.  So an
@@ -132,13 +155,6 @@ static int index_frames(const uint8_t* src, size_t n, FrameIndex& ix, bool singl
     return seen ? 0 : -1;
 }
 
-template <typename T> static size_t put(std::vector<uint8_t>& blob, size_t count)
-{
-    size_t o = (blob.size() + 15) & ~size_t(15);
-    blob.resize(o + count * sizeof(T));
-    return o;
-}
-
 static int build_descriptors(FrameIndex& ix)
 {
     for (size_t i = 0; i < ix.blocks.size(); i++) {
@@ -146,43 +162,76 @@ static int build_descriptors(FrameIndex& ix)
         if (ix.blocks[i].has_checksum) ix.bsum_ix.push_back(i);
     }
     for (size_t f = 0; f < ix.frames.size(); f++) if (ix.frames[f].has_checksum) ix.fsum_ix.push_back(f);
-    ix.n_comp = ix.comp_ix.size(); ix.n_raw = ix.raw_ix.size(); ix.n_bsum = ix.bsum_ix.size(); ix.n_fsum = ix.fsum_ix.size();
-    auto& B = ix.h_blob;
-    const size_t nf = ix.frames.size();
-    ix.o_c_soff = put<uint64_t>(B, ix.n_comp); ix.o_c_doff = put<uint64_t>(B, ix.n_comp);
-    ix.o_c_slen = put<int32_t>(B, ix.n_comp);  ix.o_c_dcap = put<int32_t>(B, ix.n_comp); ix.o_c_res = put<int32_t>(B, ix.n_comp);
-    ix.o_r_soff = put<uint64_t>(B, ix.n_raw);  ix.o_r_doff = put<uint64_t>(B, ix.n_raw); ix.o_r_len = put<int32_t>(B, ix.n_raw);
-    ix.o_h_off = put<uint64_t>(B, nf); ix.o_h_len = put<int32_t>(B, nf); ix.o_h_out = put<uint32_t>(B, nf);
-    ix.o_b_off = put<uint64_t>(B, ix.n_bsum); ix.o_b_len = put<int32_t>(B, ix.n_bsum); ix.o_b_out = put<uint32_t>(B, ix.n_bsum);
-    ix.o_f_first = put<uint32_t>(B, ix.n_fsum); ix.o_f_nblk = put<uint32_t>(B, ix.n_fsum); ix.o_f_out = put<uint32_t>(B, ix.n_fsum);
-    ix.o_k_comp = put<int32_t>(B, ix.blocks.size()); ix.o_k_rawlen = put<int32_t>(B, ix.blocks.size());
-    ix.o_k_off = put<uint64_t>(B, ix.blocks.size());
-    B.resize((B.size() + 15) & ~size_t(15));
-    uint8_t* p = B.data();
-    for (size_t k = 0; k < ix.blocks.size(); k++) ((uint64_t*)(p + ix.o_k_off))[k] = ix.blocks[k].out_off;
-    for (size_t k = 0; k < ix.n_comp; k++) ((int32_t*)(p + ix.o_k_comp))[ix.comp_ix[k]] = (int32_t)k;
-    for (size_t k = 0; k < ix.n_raw; k++) { ((int32_t*)(p + ix.o_k_comp))[ix.raw_ix[k]] = -1; ((int32_t*)(p + ix.o_k_rawlen))[ix.raw_ix[k]] = (int32_t)ix.blocks[ix.raw_ix[k]].size; }
-    for (size_t k = 0; k < ix.n_fsum; k++) {
+    size_t bytes = 0;
+    desc_view(nullptr, ix, &bytes);
+    ix.h_blob.resize(bytes);
+    const FrameDesc h = desc_view(ix.h_blob.data(), ix);
+    for (size_t k = 0; k < ix.blocks.size(); k++) h.k_off[k] = ix.blocks[k].out_off;
+    for (size_t k = 0; k < ix.fsum_ix.size(); k++) {
         const FrameRec& fr = ix.frames[ix.fsum_ix[k]];
         if (fr.first_block > 0xFFFFFFFFull || fr.nblocks > 0xFFFFFFFFull) return -10;
-        ((uint32_t*)(p + ix.o_f_first))[k] = (uint32_t)fr.first_block; ((uint32_t*)(p + ix.o_f_nblk))[k] = (uint32_t)fr.nblocks;
+        h.f_first[k] = (uint32_t)fr.first_block; h.f_nblk[k] = (uint32_t)fr.nblocks;
     }
-    for (size_t k = 0; k < ix.n_comp; k++) {
+    for (size_t k = 0; k < ix.comp_ix.size(); k++) {
         const BlockRec& b = ix.blocks[ix.comp_ix[k]];
-        ((uint64_t*)(p + ix.o_c_soff))[k] = b.src_off; ((uint64_t*)(p + ix.o_c_doff))[k] = b.out_off;
-        ((int32_t*)(p + ix.o_c_slen))[k] = (int32_t)b.size; ((int32_t*)(p + ix.o_c_dcap))[k] = (int32_t)b.cap;
+        h.k_comp[ix.comp_ix[k]] = (int32_t)k;
+        h.c_soff[k] = b.src_off; h.c_doff[k] = b.out_off; h.c_slen[k] = (int32_t)b.size; h.c_dcap[k] = (int32_t)b.cap;
     }
-    for (size_t k = 0; k < ix.n_raw; k++) {
+    for (size_t k = 0; k < ix.raw_ix.size(); k++) {
         const BlockRec& b = ix.blocks[ix.raw_ix[k]];
-        ((uint64_t*)(p + ix.o_r_soff))[k] = b.src_off; ((uint64_t*)(p + ix.o_r_doff))[k] = b.out_off; ((int32_t*)(p + ix.o_r_len))[k] = (int32_t)b.size;
+        h.k_comp[ix.raw_ix[k]] = -1; h.k_rawlen[ix.raw_ix[k]] = (int32_t)b.size;
+        h.r_soff[k] = b.src_off; h.r_doff[k] = b.out_off; h.r_len[k] = (int32_t)b.size;
     }
-    for (size_t f = 0; f < nf; f++) { ((uint64_t*)(p + ix.o_h_off))[f] = ix.frames[f].desc_off; ((int32_t*)(p + ix.o_h_len))[f] = ix.frames[f].desc_len; }
-    for (size_t k = 0; k < ix.n_bsum; k++) {
+    for (size_t f = 0; f < ix.frames.size(); f++) { h.h_off[f] = ix.frames[f].desc_off; h.h_len[f] = ix.frames[f].desc_len; }
+    for (size_t k = 0; k < ix.bsum_ix.size(); k++) {
         const BlockRec& b = ix.blocks[ix.bsum_ix[k]];
-        ((uint64_t*)(p + ix.o_b_off))[k] = b.src_off; ((int32_t*)(p + ix.o_b_len))[k] = (int32_t)b.size;
+        h.b_off[k] = b.src_off; h.b_len[k] = (int32_t)b.size;
     }
     return 0;
 }
+
+// Releases the index's device state on ix.device; the caller's current device stays current.
+static void release_device_state(FrameIndex& ix)
+{
+    if (!ix.d_blob) return;
+    int cur = -1;
+    if (cudaGetDevice(&cur) != cudaSuccess) cur = -1;
+    cudaSetDevice(ix.device);
+    cudaFree(ix.d_blob);
+    if (ix.st2) cudaStreamDestroy(ix.st2);
+    if (ix.e1) cudaEventDestroy(ix.e1);
+    if (ix.e2) cudaEventDestroy(ix.e2);
+    ix.d_blob = nullptr; ix.st2 = nullptr; ix.e1 = nullptr; ix.e2 = nullptr;
+    if (cur >= 0) cudaSetDevice(cur);
+}
+
+// Creates it on the current device `dev`: the blob's device copy, the checksum stream and its two events, all or none.
+static int create_device_state(FrameIndex& ix, int dev)
+{
+    ix.device = dev;
+    cudaError_t e = cudaMalloc(&ix.d_blob, ix.h_blob.size() + 16);
+    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&ix.st2, cudaStreamNonBlocking);
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ix.e1, cudaEventDisableTiming);
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ix.e2, cudaEventDisableTiming);
+    if (e == cudaSuccess) return 0;
+    release_device_state(ix);
+    return fail_cuda(e, "creating the frame index's device state");
+}
+
+// What one host-buffer decode holds, released when the call returns: nothing is kept between calls.
+struct HostDecode {
+    FrameIndex* ix = nullptr;
+    uint8_t *d_src = nullptr, *d_slots = nullptr, *d_tmp = nullptr;
+    cudaStream_t st = nullptr;
+    ~HostDecode()
+    {
+        if (d_tmp) cudaFree(d_tmp);
+        if (d_src) cudaFree(d_src);
+        if (d_slots) cudaFree(d_slots);
+        if (st) cudaStreamDestroy(st);
+        b200lz4f_index_free(ix);
+    }
+};
 
 } // namespace b200
 
@@ -193,7 +242,7 @@ extern "C" {
 static void* index_create(const uint8_t* src_host, size_t n, bool single, uint64_t* slot_bytes, size_t* consumed, int* err)
 {
     FrameIndex* ix = new (std::nothrow) FrameIndex();
-    if (!ix) { if (err) *err = B200LZ4_E_ARG; return nullptr; }
+    if (!ix) { const int rc = fail_arg("out of host memory"); if (err) *err = rc; return nullptr; }
     int rc = src_host ? index_frames(src_host, n, *ix, single, consumed) : -1;
     if (rc == 0) rc = build_descriptors(*ix);
     if (rc) { delete ix; if (err) *err = rc; return nullptr; }
@@ -211,7 +260,7 @@ void* b200lz4f_index_create_single(const uint8_t* src_host, size_t n, uint64_t* 
 // -1 when it declares none or when there is no frame at all; the descriptor hash is verified like nextFrameInfo does.
 int b200lz4f_expected_content_size(const uint8_t* src, size_t n, int64_t* content_size)
 {
-    if (!src || !content_size) return B200LZ4_E_ARG;
+    if (!src || !content_size) return fail_arg("null pointer");
     *content_size = -1;
     size_t ip = 0; bool seen = false;
     for (;;) {
@@ -245,8 +294,7 @@ void b200lz4f_index_free(void* index)
 {
     FrameIndex* ix = (FrameIndex*)index;
     if (!ix) return;
-    if (ix->d_blob) { cudaSetDevice(ix->device); cudaFree(ix->d_blob); }
-    if (ix->st2) { cudaSetDevice(ix->device); cudaStreamDestroy(ix->st2); cudaEventDestroy(ix->e1); cudaEventDestroy(ix->e2); }
+    release_device_state(*ix);
     delete ix;
 }
 
@@ -261,82 +309,70 @@ int64_t b200lz4f_decode_dev(void* index, const uint8_t* d_src, uint8_t* d_slots,
     FrameIndex& ix = *(FrameIndex*)index;
     cudaStream_t st = (cudaStream_t)stream;
     int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) return B200LZ4_E_NODEVICE;
-    if (ix.st2 && ix.device != dev) { cudaSetDevice(ix.device); cudaStreamDestroy(ix.st2); cudaEventDestroy(ix.e1); cudaEventDestroy(ix.e2); cudaSetDevice(dev); ix.st2 = nullptr; }
-    if (!ix.d_blob || ix.device != dev) {
-        if (ix.d_blob) { cudaSetDevice(ix.device); cudaFree(ix.d_blob); cudaSetDevice(dev); ix.d_blob = nullptr; }
-        if (cudaMalloc(&ix.d_blob, ix.h_blob.size() + 16) != cudaSuccess) return B200LZ4_E_CUDA;
-        ix.device = dev;
-    }
-    if (!ix.st2) {
-        if (cudaStreamCreateWithFlags(&ix.st2, cudaStreamNonBlocking) != cudaSuccess) { ix.st2 = nullptr; return B200LZ4_E_CUDA; }
-        if (cudaEventCreateWithFlags(&ix.e1, cudaEventDisableTiming) != cudaSuccess || cudaEventCreateWithFlags(&ix.e2, cudaEventDisableTiming) != cudaSuccess)
-            return B200LZ4_E_CUDA;
-    }
-    uint8_t* D = ix.d_blob; uint8_t* H = ix.h_blob.data();
-    const size_t nf = ix.frames.size();
-    if (cudaMemcpyAsync(D, H, ix.h_blob.size(), cudaMemcpyHostToDevice, st) != cudaSuccess) return B200LZ4_E_CUDA;
-    if (ix.n_comp && cudaMemsetAsync(D + ix.o_c_res, 0x80, ix.n_comp * 4, st) != cudaSuccess) return B200LZ4_E_CUDA;   // FRAME_RES_PENDING
+    const cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) { fail_cuda(e, "cudaGetDevice"); return B200LZ4_E_NODEVICE; }
+    if (ix.d_blob && ix.device != dev) release_device_state(ix);
+    if (!ix.d_blob) { const int rc = create_device_state(ix, dev); if (rc) return rc; }
+    const FrameDesc h = desc_view(ix.h_blob.data(), ix), d = desc_view(ix.d_blob, ix);
+    const size_t nc = ix.comp_ix.size(), nr = ix.raw_ix.size(), nbs = ix.bsum_ix.size(), nfs = ix.fsum_ix.size(), nf = ix.frames.size();
+    CK(cudaMemcpyAsync(ix.d_blob, ix.h_blob.data(), ix.h_blob.size(), cudaMemcpyHostToDevice, st));
+    if (nc) CK(cudaMemsetAsync(d.c_res, 0x80, nc * 4, st));                 // FRAME_RES_PENDING
     // 1. header + block checksums
-    g_launch_count += 1;
-    if (launch_xxh32(d_src, (uint64_t*)(D + ix.o_h_off), (int32_t*)(D + ix.o_h_len), 0, (uint32_t*)(D + ix.o_h_out), nf, st) != cudaSuccess) return B200LZ4_E_CUDA;
-    if (ix.n_bsum) {
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    CK(launch_xxh32(d_src, d.h_off, d.h_len, 0, d.h_out, nf, st));
+    if (nbs) {
         // few long payloads: one warp per stream; many short ones: one lane per buffer (xxhash.cu)
-        uint64_t sum = 0; for (size_t k = 0; k < ix.n_bsum; k++) sum += ix.blocks[ix.bsum_ix[k]].size;
-        g_launch_count += 1;
-        if ((sum / ix.n_bsum >= XXH_LONG_AVG ? launch_xxh32_long : launch_xxh32)(
-                d_src, (uint64_t*)(D + ix.o_b_off), (int32_t*)(D + ix.o_b_len), 0, (uint32_t*)(D + ix.o_b_out), ix.n_bsum, st) != cudaSuccess) return B200LZ4_E_CUDA;
+        uint64_t sum = 0; for (size_t b : ix.bsum_ix) sum += ix.blocks[b].size;
+        g_launches.fetch_add(1, std::memory_order_relaxed);
+        CK((sum / nbs >= XXH_LONG_AVG ? launch_xxh32_long : launch_xxh32)(d_src, d.b_off, d.b_len, 0, d.b_out, nbs, st));
     }
     // 2. stored blocks are copied, then every compressed block is decoded; 3. one warp per frame folds the blocks into the
     // content checksum as the decoder hands them over (second stream; the decode kernel is launched FIRST and waits for nobody)
-    if (ix.n_raw) {
-        g_launch_count += 1;
-        if (launch_gather(d_src, (uint64_t*)(D + ix.o_r_soff), (int32_t*)(D + ix.o_r_len), d_slots, (uint64_t*)(D + ix.o_r_doff), ix.n_raw, st) != cudaSuccess) return B200LZ4_E_CUDA;
+    if (nr) {
+        g_launches.fetch_add(1, std::memory_order_relaxed);
+        CK(launch_gather(d_src, d.r_soff, d.r_len, d_slots, d.r_doff, nr, st));
     }
-    if (cudaEventRecord(ix.e1, st) != cudaSuccess) return B200LZ4_E_CUDA;
-    if (ix.n_comp) {
-        BatchArgs a{ d_src, (uint64_t*)(D + ix.o_c_soff), (int32_t*)(D + ix.o_c_slen), d_slots, (uint64_t*)(D + ix.o_c_doff),
-                     (int32_t*)(D + ix.o_c_dcap), (int32_t*)(D + ix.o_c_res), ix.n_comp };
-        g_launch_count += 1;
-        if (launch_decompress_safe(a, st) != cudaSuccess) return B200LZ4_E_CUDA;
+    CK(cudaEventRecord(ix.e1, st));
+    if (nc) {
+        BatchArgs a{ d_src, d.c_soff, d.c_slen, d_slots, d.c_doff, d.c_dcap, d.c_res, nc };
+        g_launches.fetch_add(1, std::memory_order_relaxed);
+        CK(launch_decompress_safe(a, st));
     }
-    if (ix.n_fsum) {
-        if (cudaStreamWaitEvent(ix.st2, ix.e1, 0) != cudaSuccess) return B200LZ4_E_CUDA;
-        g_launch_count += 1;
-        if (launch_xxh32_frames_chained(d_slots, (uint64_t*)(D + ix.o_k_off), (uint32_t*)(D + ix.o_f_first), (uint32_t*)(D + ix.o_f_nblk),
-                                        (int32_t*)(D + ix.o_k_comp), (int32_t*)(D + ix.o_k_rawlen),
-                                        (int32_t*)(D + ix.o_c_res), (uint32_t*)(D + ix.o_f_out), ix.n_fsum, ix.st2) != cudaSuccess) return B200LZ4_E_CUDA;
-        if (cudaEventRecord(ix.e2, ix.st2) != cudaSuccess || cudaStreamWaitEvent(st, ix.e2, 0) != cudaSuccess) return B200LZ4_E_CUDA;
+    if (nfs) {
+        CK(cudaStreamWaitEvent(ix.st2, ix.e1, 0));
+        g_launches.fetch_add(1, std::memory_order_relaxed);
+        CK(launch_xxh32_frames_chained(d_slots, d.k_off, d.f_first, d.f_nblk, d.k_comp, d.k_rawlen, d.c_res, d.f_out, nfs, ix.st2));
+        CK(cudaEventRecord(ix.e2, ix.st2));
+        CK(cudaStreamWaitEvent(st, ix.e2, 0));
     }
-    if (ix.n_comp && cudaMemcpyAsync(H + ix.o_c_res, D + ix.o_c_res, ix.n_comp * 4, cudaMemcpyDeviceToHost, st) != cudaSuccess) return B200LZ4_E_CUDA;
-    if (cudaMemcpyAsync(H + ix.o_h_out, D + ix.o_h_out, nf * 4, cudaMemcpyDeviceToHost, st) != cudaSuccess) return B200LZ4_E_CUDA;
-    if (ix.n_bsum && cudaMemcpyAsync(H + ix.o_b_out, D + ix.o_b_out, ix.n_bsum * 4, cudaMemcpyDeviceToHost, st) != cudaSuccess) return B200LZ4_E_CUDA;
-    if (ix.n_fsum && cudaMemcpyAsync(H + ix.o_f_out, D + ix.o_f_out, ix.n_fsum * 4, cudaMemcpyDeviceToHost, st) != cudaSuccess) return B200LZ4_E_CUDA;
-    if (cudaStreamSynchronize(st) != cudaSuccess) return B200LZ4_E_CUDA;
+    if (nc) CK(cudaMemcpyAsync(h.c_res, d.c_res, nc * 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(h.h_out, d.h_out, nf * 4, cudaMemcpyDeviceToHost, st));
+    if (nbs) CK(cudaMemcpyAsync(h.b_out, d.b_out, nbs * 4, cudaMemcpyDeviceToHost, st));
+    if (nfs) CK(cudaMemcpyAsync(h.f_out, d.f_out, nfs * 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
 
     // the verdict, in the order the stream reader meets things: frame by frame -- descriptor hash (:208-216), then block by
     // block its checksum (:298-303) and its decode (:307-311), then at the EndMark content checksum (:266-269) and size (:270-272)
     std::vector<int32_t> bsum_of(ix.blocks.size(), -1), fsum_of(nf, -1);
-    for (size_t k = 0; k < ix.n_bsum; k++) bsum_of[ix.bsum_ix[k]] = (int32_t)k;
-    for (size_t k = 0; k < ix.n_fsum; k++) fsum_of[ix.fsum_ix[k]] = (int32_t)k;
-    const int32_t* blk_comp = (const int32_t*)(H + ix.o_k_comp);
+    for (size_t k = 0; k < nbs; k++) bsum_of[ix.bsum_ix[k]] = (int32_t)k;
+    for (size_t k = 0; k < nfs; k++) fsum_of[ix.fsum_ix[k]] = (int32_t)k;
     std::vector<int32_t> blen(ix.blocks.size());
     int64_t total = 0; bool gaps = false;
     for (size_t f = 0; f < nf; f++) {
         const FrameRec& fr = ix.frames[f];
-        if (((((uint32_t*)(H + ix.o_h_out))[f] >> 8) & 0xFF) != fr.hc_byte) return -3;
+        if (((h.h_out[f] >> 8) & 0xFF) != fr.hc_byte) return -3;
         uint64_t len = 0;
         for (size_t k = 0; k < fr.nblocks; k++) {
             const size_t b = fr.first_block + k;
             const BlockRec& br = ix.blocks[b];
-            if (bsum_of[b] >= 0 && ((uint32_t*)(H + ix.o_b_out))[bsum_of[b]] != br.checksum) return -5;
+            if (bsum_of[b] >= 0 && h.b_out[bsum_of[b]] != br.checksum) return -5;
             int32_t l = (int32_t)br.size;
-            if (!br.raw) { l = ((int32_t*)(H + ix.o_c_res))[blk_comp[b]]; if (l < 0) return -6; }   // LZ4Exception -> IOException
+            if (!br.raw) { l = h.c_res[h.k_comp[b]]; if (l < 0) return -6; }   // LZ4Exception -> IOException
             blen[b] = l;
             if (k + 1 < fr.nblocks && (uint32_t)l != fr.bs) gaps = true;          // a short block in the middle of a frame
             len += (uint64_t)l;
         }
-        if (fsum_of[f] >= 0 && ((uint32_t*)(H + ix.o_f_out))[fsum_of[f]] != fr.content_checksum) return -7;
+        if (fsum_of[f] >= 0 && h.f_out[fsum_of[f]] != fr.content_checksum) return -7;
         if (fr.has_size && fr.content_size != len) return -8;
         if (frame_off) frame_off[f] = fr.out_off;
         if (frame_len) frame_len[f] = len;
@@ -359,59 +395,52 @@ void b200lz4f_index_block_offsets(void* index, uint64_t* block_off)
 static int64_t decompress_host(const uint8_t* src, size_t n, uint8_t* dst, size_t dst_capacity, bool single, size_t* consumed)
 {
     int err = 0; uint64_t slot_bytes = 0;
-    void* index = index_create(src, n, single, &slot_bytes, consumed, &err);
-    if (!index) return err;
-    FrameIndex& ix = *(FrameIndex*)index;
-    int64_t rc = 0;
-    uint8_t *d_src = nullptr, *d_slots = nullptr;
-    cudaStream_t st = nullptr;
+    HostDecode c;
+    c.ix = (FrameIndex*)index_create(src, n, single, &slot_bytes, consumed, &err);
+    if (!c.ix) return err;
+    const FrameIndex& ix = *c.ix;
     std::vector<uint64_t> foff(ix.frames.size()), flen(ix.frames.size());
     std::vector<int32_t> blen(ix.blocks.size());
-    do {
-        if (b200lz4_device_count() <= 0) { rc = B200LZ4_E_NODEVICE; break; }
-        if (cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking) != cudaSuccess ||
-            cudaMalloc(&d_src, n + 16) != cudaSuccess || cudaMalloc(&d_slots, slot_bytes + 16) != cudaSuccess) { rc = B200LZ4_E_CUDA; break; }
-        if (cudaMemcpyAsync(d_src, src, n, cudaMemcpyHostToDevice, st) != cudaSuccess) { rc = B200LZ4_E_CUDA; break; }
-        rc = b200lz4f_decode_dev(index, d_src, d_slots, foff.data(), flen.data(), blen.data(), st);
-        if (rc < 0 && rc != -11) break;
-        // download: per frame when contiguous, else per run of blocks (short blocks in the middle of a frame)
-        uint64_t pos = 0; bool ok = true;
-        if (rc >= 0) {
-            for (size_t f = 0; f < ix.frames.size() && ok; f++) {
-                if (pos + flen[f] > dst_capacity) { rc = -9; ok = false; break; }
-                if (flen[f] && cudaMemcpyAsync(dst + pos, d_slots + foff[f], flen[f], cudaMemcpyDeviceToHost, st) != cudaSuccess) { rc = B200LZ4_E_CUDA; ok = false; }
-                pos += flen[f];
-            }
-        } else {
-            // short blocks in mid-frame (everything is verified already): the device packs the blocks, one copy brings them back
-            rc = 0;
-            const size_t nb = ix.blocks.size();
-            std::vector<uint64_t> from(nb), to(nb);
-            for (size_t b = 0; b < nb; b++) { from[b] = ix.blocks[b].out_off; to[b] = pos; pos += (uint64_t)blen[b]; }
-            if (pos > dst_capacity) { rc = -9; ok = false; }
-            uint8_t* d_tmp = nullptr;
-            const size_t o_to = (nb * 8 + 15) & ~size_t(15), o_len = 2 * o_to, o_out = (o_len + nb * 4 + 15) & ~size_t(15);
-            if (ok && pos) {
-                if (cudaMalloc(&d_tmp, o_out + pos + 16) != cudaSuccess) { rc = B200LZ4_E_CUDA; ok = false; d_tmp = nullptr; }
-                if (ok && (cudaMemcpyAsync(d_tmp, from.data(), nb * 8, cudaMemcpyHostToDevice, st) != cudaSuccess ||
-                           cudaMemcpyAsync(d_tmp + o_to, to.data(), nb * 8, cudaMemcpyHostToDevice, st) != cudaSuccess ||
-                           cudaMemcpyAsync(d_tmp + o_len, blen.data(), nb * 4, cudaMemcpyHostToDevice, st) != cudaSuccess)) { rc = B200LZ4_E_CUDA; ok = false; }
-                if (ok) {
-                    g_launch_count += 1;
-                    if (launch_gather(d_slots, (uint64_t*)d_tmp, (int32_t*)(d_tmp + o_len), d_tmp + o_out, (uint64_t*)(d_tmp + o_to), nb, st) != cudaSuccess ||
-                        cudaMemcpyAsync(dst, d_tmp + o_out, pos, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-                        cudaStreamSynchronize(st) != cudaSuccess) { rc = B200LZ4_E_CUDA; ok = false; }
-                }
-            }
-            if (d_tmp) cudaFree(d_tmp);
+    if (b200lz4_device_count() <= 0) return B200LZ4_E_NODEVICE;           // a failed query has set the message
+    CK(cudaStreamCreateWithFlags(&c.st, cudaStreamNonBlocking));
+    CK(cudaMalloc(&c.d_src, n + 16));
+    CK(cudaMalloc(&c.d_slots, slot_bytes + 16));
+    CK(cudaMemcpyAsync(c.d_src, src, n, cudaMemcpyHostToDevice, c.st));
+    const int64_t rc = b200lz4f_decode_dev(c.ix, c.d_src, c.d_slots, foff.data(), flen.data(), blen.data(), c.st);
+    if (rc < 0 && rc != -11) return rc;
+    uint64_t pos = 0;
+    if (rc >= 0) {
+        // contiguous frames: one copy per frame
+        for (size_t f = 0; f < ix.frames.size(); f++) {
+            if (pos + flen[f] > dst_capacity) return -9;
+            if (flen[f]) CK(cudaMemcpyAsync(dst + pos, c.d_slots + foff[f], flen[f], cudaMemcpyDeviceToHost, c.st));
+            pos += flen[f];
         }
-        if (ok) { if (cudaStreamSynchronize(st) != cudaSuccess) rc = B200LZ4_E_CUDA; else rc = (int64_t)pos; }
-    } while (0);
-    if (d_src) cudaFree(d_src);
-    if (d_slots) cudaFree(d_slots);
-    if (st) cudaStreamDestroy(st);
-    b200lz4f_index_free(index);
-    return rc;
+    } else {
+        // short blocks in mid-frame (everything is verified already): the device packs the blocks, one copy brings them back
+        const size_t nb = ix.blocks.size();
+        std::vector<uint64_t> from(nb), to(nb);
+        for (size_t b = 0; b < nb; b++) { from[b] = ix.blocks[b].out_off; to[b] = pos; pos += (uint64_t)blen[b]; }
+        if (pos > dst_capacity) return -9;
+        if (pos) {
+            // d_tmp: [from | to] u64, [len] i32, then the packed bytes; every part starts on 16 bytes
+            const size_t offs_bytes = (nb * 8 + 15) & ~size_t(15), lens_bytes = (nb * 4 + 15) & ~size_t(15);
+            CK(cudaMalloc(&c.d_tmp, 2 * offs_bytes + lens_bytes + pos + 16));
+            uint64_t* const d_from = (uint64_t*)c.d_tmp;
+            uint64_t* const d_to = (uint64_t*)(c.d_tmp + offs_bytes);
+            int32_t* const d_len = (int32_t*)(c.d_tmp + 2 * offs_bytes);
+            uint8_t* const d_out = c.d_tmp + 2 * offs_bytes + lens_bytes;
+            CK(cudaMemcpyAsync(d_from, from.data(), nb * 8, cudaMemcpyHostToDevice, c.st));
+            CK(cudaMemcpyAsync(d_to, to.data(), nb * 8, cudaMemcpyHostToDevice, c.st));
+            CK(cudaMemcpyAsync(d_len, blen.data(), nb * 4, cudaMemcpyHostToDevice, c.st));
+            g_launches.fetch_add(1, std::memory_order_relaxed);
+            CK(launch_gather(c.d_slots, d_from, d_len, d_out, d_to, nb, c.st));
+            CK(cudaMemcpyAsync(dst, d_out, pos, cudaMemcpyDeviceToHost, c.st));
+            CK(cudaStreamSynchronize(c.st));
+        }
+    }
+    CK(cudaStreamSynchronize(c.st));
+    return (int64_t)pos;
 }
 
 int64_t b200lz4f_decompress_host(const uint8_t* src, size_t n, uint8_t* dst, size_t dst_capacity)

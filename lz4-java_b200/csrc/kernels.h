@@ -61,6 +61,12 @@ cudaError_t launch_compact(const uint8_t* slots, const uint64_t* slot_off, const
 static inline uint64_t lz4_bound(int32_t len) { const uint64_t n = len > 0 ? (uint64_t)len : 0; return n + n / 255 + 16; }
 static inline uint64_t lz4_slot_bytes(int32_t len) { return (lz4_bound(len) + 15) & ~uint64_t(15); }
 
-extern std::atomic<unsigned long long> g_launch_count;      // launches made outside capi.cu (frame / container calls, any thread)
+// Host-side state of the library, defined in capi.cu and shared by the host files (capi.cu, frame.cu, containers.cu).
+extern std::atomic<unsigned long long> g_launches;          // kernel launches of every entry point, any thread (b200lz4_launch_count)
+// Record what went wrong for b200lz4_last_error / b200lz4_last_status and return the code: B200LZ4_E_NODEVICE or _E_CUDA
+// (fail_cuda), B200LZ4_E_ARG (fail_arg).
+int fail_cuda(cudaError_t e, const char* where);
+int fail_arg(const char* what);
+#define CK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return b200::fail_cuda(e_, #call); } while (0)
 
 } // namespace b200

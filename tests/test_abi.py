@@ -1,5 +1,6 @@
 """C-ABI checks that need no GPU: the library loads, exports every symbol include/b200lz4.h declares,
 pure-arithmetic entry points work, and compute entry points fail LOUDLY (no CPU fallback) without a device."""
+import ctypes
 import os
 import re
 
@@ -44,7 +45,7 @@ def _no_gpu(b200):
     return b200._native.lib().b200lz4_device_count() < 0
 
 
-def test_no_device_is_loud(b200):
+def test_no_device_is_loud(b200, port):
     """without a usable GPU the product raises; it never computes on the CPU"""
     if not _no_gpu(b200):
         pytest.skip("a CUDA device is present")
@@ -66,6 +67,24 @@ def test_no_device_is_loud(b200):
         b200.xxhash.XXHash32().hash(src.tobytes(), 0, 100, 0)
     with pytest.raises(b200.B200Error):
         b200.xxhash.XXHash64().hash(src.tobytes(), 0, 100, 0)
+    # the frame and container calls return the same code, and leave their own status and message behind (not an earlier
+    # call's: each check starts from an argument error's); the frame writer writes no frame with a missing checksum
+    E = b200._native.E_NODEVICE
+    out = np.zeros(64, dtype=np.uint8)
+    frame = np.frombuffer(port.frame_compress(b"a small frame", 4, 1), dtype=np.uint8)
+    size = ctypes.c_int64(0)
+    calls = [lambda flags=flags: lib.b200lz4f_compress_host(src.ctypes.data, 0, out.ctypes.data, len(out), 4, flags) for flags in (0, 1, 5)]
+    calls += [lambda: lib.b200lz4f_decompress_host(frame.ctypes.data, len(frame), out.ctypes.data, len(out)),
+              lambda: lib.b200lz4f_expected_content_size(frame.ctypes.data, len(frame), ctypes.byref(size)),
+              lambda: lib.b200lz4block_compress_host(src.ctypes.data, 1, out.ctypes.data, len(out), 1 << 16)]
+    for i, call in enumerate(calls):
+        lib.b200xxh32(src.ctypes.data, 1 << 31, 0)
+        assert lib.b200lz4_last_status() == b200._native.E_ARG
+        assert call() == E, i
+        msg = b200._native.last_error()
+        assert lib.b200lz4_last_status() == E and msg and "invalid argument" not in msg, (i, msg)
+    with pytest.raises(b200.B200Error):
+        b200.compress_frame(b"")
 
 
 def test_product_does_not_import_oracle():

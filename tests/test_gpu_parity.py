@@ -1231,6 +1231,37 @@ def test_frames_written_with_flush(b200, port):
     d_bad = M.up(np.concatenate([bad, np.zeros(64, dtype=np.uint8)]))
     assert N.lib().b200lz4f_decode_dev(ix2, M.ptr(d_bad), M.ptr(d_slots), None, None, None, None) == -7
     N.lib().b200lz4f_index_free(ix); N.lib().b200lz4f_index_free(ix2)
+    # the host path on a gapped frame with a stored block makes six launches, all counted: descriptor hash, block hashes,
+    # stored-block gather, decode, chained content hash, and the gather that packs the blocks
+    f = _frame_of_pieces(port, pieces, 4, content_checksum=True, block_checksum=True, stored={1})
+    N.lib().b200lz4_launch_count_reset()
+    assert b200.decompress_frames(f, sum(map(len, pieces))) == b"".join(pieces)
+    assert N.lib().b200lz4_launch_count() == 6
+
+
+def test_frame_index_free_keeps_the_current_device(b200, port):
+    """an index decoded on GPU 0 and freed while GPU 1 is current releases its device state on GPU 0 and leaves GPU 1 current"""
+    import ctypes
+    M = _DevMem()
+    if M.sim or M.torch.cuda.device_count() < 2:
+        pytest.skip("needs two GPUs")
+    L = b200._native.lib()
+    data = port.datagen(200000, 0.5, 0.0, 3).tobytes()
+    f = np.frombuffer(port.frame_compress(data, 4, 3), dtype=np.uint8)
+    slot, err = ctypes.c_uint64(0), ctypes.c_int(0)
+    ix = L.b200lz4f_index_create(f.ctypes.data, len(f), ctypes.byref(slot), ctypes.byref(err))
+    assert ix and err.value == 0
+    try:
+        M.torch.cuda.set_device(0)
+        d_src, d_slots = M.up(np.concatenate([f, np.zeros(64, dtype=np.uint8)]), 0), M.zeros(slot.value + 64, 0)
+        assert L.b200lz4f_decode_dev(ix, M.ptr(d_src), M.ptr(d_slots), None, None, None, None) == len(data)
+        assert M.down(d_slots)[:len(data)].tobytes() == data
+        M.zeros(16, 1)                                              # GPU 1 has a context, so the current device is CUDA's own
+        M.torch.cuda.set_device(1)
+        L.b200lz4f_index_free(ix)
+        assert M.torch.cuda.current_device() == 1
+    finally:
+        M.torch.cuda.set_device(0)
 
 
 def test_container_writers_with_the_high_compressor(b200, port):
